@@ -1,7 +1,7 @@
 """bench.py -- the BASELINE metric: frames/sec at 1080p with depth_anything (ViT-L) AND flow_raft (12 GRU iterations,
 forward + backward flow) computed for every frame of a synthetic clip, at N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one chunk of FRAMES_PER_STEP consecutive 1080p frames per GPU pushed through both bands, the way
@@ -20,8 +20,9 @@ the barrier and the max-over-ranks of the timings.
                convs, RAFT encoder / update-block convs): algorithmic FLOP of all its launches / their CUDA-event time,
                vs the measured sustained bf16 peak; `groups` breaks it down and adds the attention kernel and the
                HBM-bound RAFT correlation build (vs the measured copy bandwidth)
-  cpu_baseline / --impl reference : the oracle port of the reference's CPU fp32 path (oracle/da.py + oracle/raft.py; the
-               Python reference itself cannot travel to the GPU box) on the host cores, on a bounded sample of frames
+  cpu_baseline / --impl reference : the oracle port of the reference's CPU fp32 path (oracle/da.py + oracle/raft.py) on
+               the host cores: one frame for cpu_baseline, one frame per --steps step for --impl reference
+  --dump-outputs DIR : what the last timed e2e step handed back to the caller, as .npy files (see dump_outputs)
 """
 import argparse
 import json
@@ -99,6 +100,21 @@ def make_frames(n, h, w, start):
     return frames
 
 
+DUMP_SAMPLE = 1 << 21   # elements kept of an output larger than this: 3 frame stacks x 8 MB of float32, under 64 MB in all
+
+
+def dump_outputs(directory, arrays):
+    """Write each array as <directory>/<name>.npy in float32.  An array larger than DUMP_SAMPLE elements is replaced by a
+    fixed sample of its flattened elements (sorted indices drawn from a generator seeded with 0), so two builds run with
+    the same arguments can be compared output for output."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).integers(0, a.size, DUMP_SAMPLE))]
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float32))
+
+
 def cpu_threads():
     """torch CPU scales to ~32 threads on the GPU box's host (measured with tools/cpu_threads.py: 8 thr 7.4 s/frame,
     16: 6.3, 32: 6.0, 64: 7.7, 128: 41 s/frame) -- use the optimum, and say so."""
@@ -134,7 +150,7 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     cores = cpu_threads()
-    steps = max(1, min(args.steps, 3))  # bounded: ~15-40 s of CPU work per 1080p frame (ViT-L + RAFT)
+    steps = args.steps  # one 1080p frame per step: ~15-40 s of CPU work each (ViT-L + RAFT)
     fps, dt = cpu_reference_step(steps, cores)
     out = {
         "impl": "reference", "metric": "frames/sec at 1080p (depth_anything+flow_raft)", "value": fps, "unit": "frames/s",
@@ -299,9 +315,13 @@ def run_b200(args, rank, local_rank, world):
     out_flow = {"fwd_rgb": pinned_empty((FRAMES_PER_STEP, hs, ws, 3), np.uint8),
                 "bwd_rgb": pinned_empty((FRAMES_PER_STEP, hs, ws, 3), np.uint8)}
 
+    last = {}   # what the caller received from the most recent e2e step (for --dump-outputs)
+
     def e2e_step(cont):
-        da.infer_clip(clip, pass_frames=BATCH, out_rgb=out_depth_rgb)
+        rgb, mins, maxs, _ = da.infer_clip(clip, pass_frames=BATCH, out_rgb=out_depth_rgb)
         r = raft.infer_clip(clip, continue_clip=cont, want_flow=False, want_rgb=True, out=out_flow)
+        last.update(depth_rgb=rgb, depth_min=mins, depth_max=maxs, flow_fwd_rgb=r["fwd_rgb"], flow_bwd_rgb=r["bwd_rgb"],
+                    flow_max_fwd=r["max_fwd"], flow_max_bwd=r["max_bwd"])
         return r["pairs"]
 
     # ---------------- e2e: public API, H2D + D2H inside the timed region.  The clip continues from step to step (every
@@ -406,6 +426,8 @@ def run_b200(args, rank, local_rank, world):
                                              f"iterations, fwd+bwd, + process_flow), torch CPU fp32, {cores} threads of "
                                              f"{os.cpu_count()} host cores (the measured optimum), {dt:.1f} s"}
         print(json.dumps(out), flush=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     da.close()
     raft.close()
     if dist is not None:
@@ -420,7 +442,15 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary workloads (other bands)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last end-to-end step returned (depth and flow frames, "
+                         "per-frame scalars) as DIR/<name>.npy in float32; frame stacks are a fixed seeded sample; "
+                         "rank 0's frames when --gpus > 1")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

@@ -16,3 +16,14 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN
+
+
+@pytest.fixture
+def recorded_threads():
+    """Run on the 8 torch intra-op threads the bit-exact CPU fixtures were recorded with (on an AVX-512 host).  oneDNN
+    splits fp32 convolution sums by thread count, so a replay on another count differs in the last bits."""
+    import torch
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)

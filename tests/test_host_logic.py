@@ -75,3 +75,25 @@ def test_mask_band_precision_flag_selects_the_engine_variant():
     for flag, variant in (("exact", "r101-exact"), ("mixed", "r101"), ("fast", "r101-fast")):
         a = p.parse_args(["-i", "x.png", "--precision", flag])
         assert "r101" + {"fast": "-fast", "exact": "-exact"}.get(a.precision, "") == variant
+
+
+def test_bench_dump_outputs_is_bounded_and_reproducible(tmp_path):
+    """bench.py --dump-outputs at the benchmark's own output shapes: float32 .npy files, 64 MB at most in all, the same
+    sample from run to run, small arrays kept whole."""
+    import bench
+    n, hs, ws = bench.FRAMES_PER_STEP, int(np.rint(bench.H * bench.RAFT_SCALE)), int(np.rint(bench.W * bench.RAFT_SCALE))
+    rng = np.random.default_rng(1)
+    arrays = {"depth_rgb": rng.integers(0, 256, (n, bench.H, bench.W, 3), dtype=np.uint8),
+              "flow_fwd_rgb": rng.integers(0, 256, (n, hs, ws, 3), dtype=np.uint8),
+              "flow_bwd_rgb": rng.integers(0, 256, (n, hs, ws, 3), dtype=np.uint8),
+              "depth_min": rng.standard_normal(n).astype(np.float32), "flow_max_fwd": rng.standard_normal(n).astype(np.float32)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(k + ".npy" for k in arrays)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / "a" / "depth_min.npy"), arrays["depth_min"])
+    assert np.load(tmp_path / "a" / "depth_rgb.npy").size == bench.DUMP_SAMPLE

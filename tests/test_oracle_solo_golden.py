@@ -10,7 +10,7 @@ from oracle import solo as osolo
 from prisma_b200.seeded_weights import SOLO_CONFIGS, make_solo_weights
 
 
-def test_solo_oracle_matches_vendored_mmdet_fixture(golden_dir):
+def test_solo_oracle_matches_vendored_mmdet_fixture(golden_dir, recorded_threads):
     g = np.load(os.path.join(golden_dir, "solo_tiny_head.npz"))
     sd = make_solo_weights("tiny", 0)
     c = SOLO_CONFIGS["tiny"]

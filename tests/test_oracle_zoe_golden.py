@@ -9,7 +9,7 @@ from oracle import zoe as ozoe
 from prisma_b200.seeded_weights import make_zoe_weights
 
 
-def test_zoe_oracle_matches_reference_fixture(golden_dir):
+def test_zoe_oracle_matches_reference_fixture(golden_dir, recorded_threads):
     g = np.load(os.path.join(golden_dir, "zoe_vits_240x320.npz"))
     sd = make_zoe_weights("vits", 0)
     taps = {}
