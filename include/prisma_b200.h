@@ -212,7 +212,7 @@ int prisma_net_size(const char* band, int w, int h, int* wn, int* hn);
 int prisma_debug_gemm(int device, const float* A, const float* W, const float* bias, float* D, int M, int N, int K,
                       int act, int force_bn, int iters, float* ms_out);
 /* The same product through the 3xTF32 path of the mask band (kind::tf32 tensor-core MMAs on [hi | lo] splits of both
- * operands: fp32-class products, ~1e-6 relative): D = A W^T + bias, all fp32.                                  */
+ * operands: fp32-class products, ~1e-6 relative): D = A W^T + bias, all fp32.  force_bn: 0 = auto, else 32/64/128.    */
 int prisma_debug_gemm_tf32x3(int device, const float* A, const float* W, const float* bias, float* D, int M, int N, int K,
                              int force_bn, int iters, float* ms_out);
 /* 3x3 (kh x kw) stride-1 'same' convolution, NHWC fp32 host in/out, through the shifted-row GEMM.           */

@@ -35,30 +35,11 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
-// exp2 on the FMA / ALU pipes for a fraction of the elements: Cody-Waite split x = n + f, f in [-0.5, 0.5], 2^f by a degree-3
-// minimax polynomial (max relative error 7.6e-5, well below the 4.9e-4 rounding of the fp16 probability it becomes), 2^n by
-// adding n to the exponent field.  x <= 8 here (lazy-rescale slack).  MEASURED AND LEFT OFF (B200, 2443 tokens, 192 heads):
-// none 643 TFLOP/s, every 4th element 636, every 3rd 619, every 2nd 550 -- with two in-order softmax warps per scheduler the
-// kernel is bound by issue slots and dependency latency, not by the exp pipe's 16 / clk, so nine instructions instead of two
-// per element lose.  -DPRISMA_ATTN_POLY=n builds the variant.
-#ifndef PRISMA_ATTN_POLY
-#define PRISMA_ATTN_POLY 0   // every PRISMA_ATTN_POLY-th element of a chunk takes the polynomial (0: none)
-#endif
-__device__ __forceinline__ float ex2_poly3(float x) {
-  x = fmaxf(x, -125.f);
-  const float r = x + 12582912.f;        // 1.5 * 2^23: round(x) lands in the low mantissa bits
-  const float f = x - (r - 12582912.f);
-  float p = fmaf(0.05520550534f, f, 0.2426139712f);
-  p = fmaf(p, f, 0.6932547688f);
-  p = fmaf(p, f, 0.9999276996f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(r) << 23));
-}
-__device__ __forceinline__ float att_ex2(float x, int i) {
-#if PRISMA_ATTN_POLY > 0
-  if (i % PRISMA_ATTN_POLY == PRISMA_ATTN_POLY - 1) return ex2_poly3(x);
-#endif
-  return ex2_approx(x);
-}
+// Every exp2 of the softmax runs on the MUFU pipe.  Measured against moving a fraction of the elements to the FMA / ALU pipes
+// (Cody-Waite split x = n + f, 2^f by a degree-3 minimax polynomial, 2^n by adding n to the exponent field; B200, 2443 tokens,
+// 192 heads): none 643 TFLOP/s, every 4th element 636, every 3rd 619, every 2nd 550 -- with two in-order softmax warps per
+// scheduler the kernel is bound by issue slots and dependency latency, not by the exp pipe's 16 / clk, so nine instructions
+// instead of two per element lose.
 
 // 32 scores -> 32 probabilities, in place; fp16 pairs to pk[16], their sum to four partial sums.  nvalid < 32: the rest are 0.
 template <bool PARTIAL>
@@ -90,7 +71,7 @@ __device__ __forceinline__ void att_exp_tile(uint32_t* v, float mscaled, uint32_
                                              float& s3) {
   const float LOG2E = 1.4426950408889634f;
 #pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(att_ex2(fmaf(__uint_as_float(v[i]), LOG2E, -mscaled), i));
+  for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(ex2_approx(fmaf(__uint_as_float(v[i]), LOG2E, -mscaled)));
 #pragma unroll
   for (int c = 0; c < 4; ++c) {
     uint32_t* e = v + c * 32;
@@ -104,7 +85,7 @@ __device__ __forceinline__ void att_exp_tile(uint32_t* v, float mscaled, uint32_
     for (int g = 0; g < 4; ++g) {
       if (c + 1 < 4) {
 #pragma unroll
-        for (int i = 0; i < 8; ++i) nx[g * 8 + i] = __float_as_uint(att_ex2(__uint_as_float(nx[g * 8 + i]), g * 8 + i));
+        for (int i = 0; i < 8; ++i) nx[g * 8 + i] = __float_as_uint(ex2_approx(__uint_as_float(nx[g * 8 + i])));
       }
       const uint32_t* q = e + g * 8;
       s0 += __uint_as_float(q[0]) + __uint_as_float(q[4]); s1 += __uint_as_float(q[1]) + __uint_as_float(q[5]);

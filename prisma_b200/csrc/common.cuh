@@ -69,18 +69,6 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 
-// ---- programmatic dependent launch ------------------------------------------------------------------
-// Every kernel of a band's pass begins with pdl_prologue(): (1) griddepcontrol.launch_dependents lets the NEXT kernel of the
-// stream / graph be scheduled as soon as every CTA of this one has started -- its CTAs become resident where resources
-// allow, run their own prologue (barrier init, TMEM allocation, descriptor prefetch) and block in (2) griddepcontrol.wait,
-// which returns when the PREVIOUS kernel has completed and its writes are visible.  Nothing touches global memory before
-// the wait, so the dependency chain is the stream order, only the ~2-4 us of launch latency and prologue per kernel
-// overlap the predecessor's tail (a RAFT pass is ~330 kernels of 5-40 us).  Both instructions are no-ops for a kernel
-// launched without the programmatic-serialization attribute (pdl_launch below sets it).
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_prologue() { pdl_launch_dependents(); pdl_wait(); }
-
 // ---- mbarrier ---------------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
@@ -347,22 +335,5 @@ int make_tmap_2d_f16(CUtensorMap* out, const void* base, uint64_t cols, uint64_t
 // the same for an fp32 tensor (box_cols must be 32 -> 128-byte inner box): the destination of the TMA-store epilogue
 int make_tmap_2d_f32(CUtensorMap* out, const void* base, uint64_t cols, uint64_t rows, uint64_t pitch_elems,
                      uint32_t box_cols, uint32_t box_rows);
-
-// Launch with the programmatic-stream-serialization attribute when PRISMA_PDL=1 (default: a plain launch; see gemm.cu for the
-// measurement that turned it off).
-bool pdl_enabled();
-#ifdef __CUDACC__
-template <typename... KArgs, typename... Args>
-inline cudaError_t pdl_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-#endif
 
 }  // namespace prisma

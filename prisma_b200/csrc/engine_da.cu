@@ -504,23 +504,21 @@ int DepthEngine::build_plan(int H, int W, int Bt) {
     const float* x = b.x; __half* ln = b.ln; const int T_ = BT, D_ = D;
     add(G_LN, "ln1", [=](cudaStream_t s) { return layernorm_f16(x, k.n1w, k.n1b, ln, T_, D_, 1e-6f, s); });
     // qkv and fc1 write dense fp16 rows: bias (+ GELU) in the row-per-lane registers, then TMA bulk stores -- no staging
-    // read-back, no per-lane global stores (the epilogue, not the MMA, paces these launches: DESIGN 4.1).  PRISMA_DA_TMA_STORE=0: off
-    static const bool tma_ep = [] { const char* e = getenv("PRISMA_DA_TMA_STORE"); return !(e && e[0] == '0'); }();
-    { GemmEpilogue ep; ep.bias = k.qkv_b; ep.out_f16 = b.qkv; ep.out_f16_ld = 3 * D; ep.tma_store = tma_ep && BT >= 1024;
+    // read-back, no per-lane global stores (the epilogue, not the MMA, paces these launches: DESIGN 4.1)
+    { GemmEpilogue ep; ep.bias = k.qkv_b; ep.out_f16 = b.qkv; ep.out_f16_ld = 3 * D; ep.tma_store = BT >= 1024;
       PRISMA_TRY(add_gemm(G_LINEAR, "qkv", b.ln, BT, D, D, k.qkv_w, BT, 3 * D, 1, zero_off, ep, 2.0 * BT * 3.0 * D * D)); }
     work_attn += att.flops;
     add(G_ATTN, "attention", [att](cudaStream_t s) { return attention_run(att, s); });
     // proj / fc2 update the fp32 token stream in place: gamma (acc + bias) is staged and added by TMA reduce-add stores
-    // (the add happens in the L2; the epilogue reads nothing).  PRISMA_DA_TMA_REDUCE=0: the register path
-    static const bool tma_red = [] { const char* e = getenv("PRISMA_DA_TMA_REDUCE"); return !(e && e[0] == '0'); }();
+    // (the add happens in the L2; the epilogue reads nothing)
     { GemmEpilogue ep; ep.bias = k.proj_b; ep.gamma = k.g1; ep.res_f32 = b.x; ep.res_f32_ld = D; ep.out_f32 = b.x; ep.out_f32_ld = D;
-      ep.tma_store = tma_red && BT >= 1024;
+      ep.tma_store = BT >= 1024;
       PRISMA_TRY(add_gemm(G_LINEAR, "proj", b.attn, BT, D, D, k.proj_w, BT, D, 1, zero_off, ep, 2.0 * BT * (double)D * D)); }
     add(G_LN, "ln2", [=](cudaStream_t s) { return layernorm_f16(x, k.n2w, k.n2b, ln, T_, D_, 1e-6f, s); });
-    { GemmEpilogue ep; ep.bias = k.fc1_b; ep.act = 1; ep.out_f16 = b.hid; ep.out_f16_ld = 4 * D; ep.tma_store = tma_ep && BT >= 1024;
+    { GemmEpilogue ep; ep.bias = k.fc1_b; ep.act = 1; ep.out_f16 = b.hid; ep.out_f16_ld = 4 * D; ep.tma_store = BT >= 1024;
       PRISMA_TRY(add_gemm(G_LINEAR, "fc1", b.ln, BT, D, D, k.fc1_w, BT, 4 * D, 1, zero_off, ep, 2.0 * BT * 4.0 * D * D)); }
     { GemmEpilogue ep; ep.bias = k.fc2_b; ep.gamma = k.g2; ep.res_f32 = b.x; ep.res_f32_ld = D; ep.out_f32 = b.x; ep.out_f32_ld = D;
-      ep.tma_store = tma_red && BT >= 1024;
+      ep.tma_store = BT >= 1024;
       PRISMA_TRY(add_gemm(G_LINEAR, "fc2", b.hid, BT, 4 * D, 4 * D, k.fc2_w, BT, D, 1, zero_off, ep, 2.0 * BT * 4.0 * D * D)); }
     if (!midas && i >= depth - 4) {
       __half* f = b.feat[i - (depth - 4)];

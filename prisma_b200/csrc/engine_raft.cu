@@ -469,8 +469,8 @@ int RaftEngine::build_plan(int H, int W, double scale, int iters_) {
       add("reuse_prev", [=](cudaStream_t s) {
         const size_t n = (size_t)c->rows_pad * c->C * sizeof(__half);
         PRISMA_CUDA_OK(cudaMemcpyAsync(c->feat, c->feat + (size_t)NP * c->rows_pad * c->C, n, cudaMemcpyDeviceToDevice, s));
-        const size_t pn = (size_t)c->rows123_pad * c->C * c->pw * sizeof(__half);
-        PRISMA_CUDA_OK(cudaMemcpyAsync(c->pool123, c->pool123 + (size_t)NP * c->rows123_pad * c->C * c->pw, pn, cudaMemcpyDeviceToDevice, s));
+        const size_t pn = (size_t)c->rows123_pad * c->C * sizeof(__half);
+        PRISMA_CUDA_OK(cudaMemcpyAsync(c->pool123, c->pool123 + (size_t)NP * c->rows123_pad * c->C, pn, cudaMemcpyDeviceToDevice, s));
         PRISMA_CUDA_OK(cudaMemcpyAsync(cn, reinterpret_cast<const char*>(cn) + NP * cn_n, cn_n, cudaMemcpyDeviceToDevice, s));
         PRISMA_CUDA_OK(cudaMemcpyAsync(rsz, rsz + NP * rbytes, rbytes, cudaMemcpyDeviceToDevice, s));
         return 0;
@@ -540,16 +540,13 @@ int RaftEngine::build_plan(int H, int W, double scale, int iters_) {
   PRISMA_TRY(new_map(&f1, B, H8, W8, 128, 2));
   __half* f1_cols = nullptr;
   PRISMA_TRY(r_alloc(plan_allocs, &f1_cols, (size_t)B * H8 * W8 * 256));
-  float *zr_f = nullptr, *q_f = nullptr;  // gates in fp32, padded-row layout of the pad-2 maps
-  static const bool fuse_gru = [] { const char* e = getenv("PRISMA_RAFT_FUSE_GRU"); return !(e && e[0] == '0'); }();
+  float* zr_f = nullptr;  // gates in fp32, padded-row layout of the pad-2 maps
   PRISMA_TRY(r_alloc(plan_allocs, &zr_f, (size_t)hx.rows() * 256));
-  PRISMA_TRY(r_alloc(plan_allocs, &q_f, (size_t)hx.rows() * 128));
   PRISMA_TRY(new_map(&fh, B, H8, W8, 256, 2));
   float* fh2_u = nullptr;
   PRISMA_TRY(r_alloc(plan_allocs, &fh2_u, (size_t)hx.rows() * 32));
   PRISMA_TRY(new_map(&mk, B, H8, W8, 256, 2));
   PRISMA_TRY(r_alloc(plan_allocs, &b.mask, (size_t)hx.rows() * 576));
-  const long long rows = hx.rows();
   for (int it = 0; it < iters; ++it) {
     {
       FlowCorr* c = corr; const float* c1p = b.coords1; __half* dst = corrf.p; const int wp = corrf.Wp(), ir = (int)corrf.img_rows();
@@ -583,24 +580,13 @@ int RaftEngine::build_plan(int H, int W, double scale, int iters_) {
       add("flow_cols", [=](cudaStream_t s) { return raft_flow_cols(c0, c1p, B, h8, w8, 2, ir8, hxp, rhp, s); });
     }
     for (int pass = 0; pass < 2; ++pass) {  // SepConvGRU horizontal then vertical (update.py:45-60)
-      if (fuse_gru) {
-        // gate arithmetic in the conv epilogues: r * h -> the q conv's operand; h' = (1 - z) h + z q -> fp32 master + operand copy
-        { GemmEpilogue ep; ep.act = 3; ep.out_f32 = zr_f; ep.out_f32_ld = 256;
-          ep.gru = 1; ep.gru_h = b.h_master; ep.gru_rh = rhx.p; ep.gru_rh_ld = 384;
-          PRISMA_TRY(add_conv("gru_zr", hx, 0, w.zr[pass], ep, 1)); }
-        { GemmEpilogue ep; ep.act = 4; ep.out_f32 = b.h_master; ep.out_f32_ld = 128; ep.out_f16 = hx.p; ep.out_f16_ld = 384;
-          ep.gru = 2; ep.gru_h = b.h_master; ep.gru_z = zr_f;
-          PRISMA_TRY(add_conv("gru_q", rhx, 0, w.q[pass], ep, 1)); }
-      } else {
-        { GemmEpilogue ep; ep.act = 3; ep.out_f32 = zr_f; ep.out_f32_ld = 256;
-          PRISMA_TRY(add_conv("gru_zr", hx, 0, w.zr[pass], ep, 1)); }
-        { const float* z = zr_f; const float* hm = b.h_master; __half* rhp = rhx.p;
-          add("gru_rh", [=](cudaStream_t s) { return raft_gru_rh(z, hm, rhp, rows, s); }); }
-        { GemmEpilogue ep; ep.act = 4; ep.out_f32 = q_f; ep.out_f32_ld = 128;
-          PRISMA_TRY(add_conv("gru_q", rhx, 0, w.q[pass], ep, 1)); }
-        { const float* z = zr_f; const float* qq = q_f; float* hm = b.h_master; __half* hxp = hx.p;
-          add("gru_update", [=](cudaStream_t s) { return raft_gru_update(z, qq, hm, hxp, rows, s); }); }
-      }
+      // gate arithmetic in the conv epilogues: r * h -> the q conv's operand; h' = (1 - z) h + z q -> fp32 master + operand copy
+      { GemmEpilogue ep; ep.act = 3; ep.out_f32 = zr_f; ep.out_f32_ld = 256;
+        ep.gru = 1; ep.gru_h = b.h_master; ep.gru_rh = rhx.p; ep.gru_rh_ld = 384;
+        PRISMA_TRY(add_conv("gru_zr", hx, 0, w.zr[pass], ep, 1)); }
+      { GemmEpilogue ep; ep.act = 4; ep.out_f32 = b.h_master; ep.out_f32_ld = 128; ep.out_f16 = hx.p; ep.out_f16_ld = 384;
+        ep.gru = 2; ep.gru_h = b.h_master; ep.gru_z = zr_f;
+        PRISMA_TRY(add_conv("gru_q", rhx, 0, w.q[pass], ep, 1)); }
     }
     { GemmEpilogue ep; ep.act = 2; ep.out_f16 = fh.p; ep.out_f16_ld = 256;            // flow head
       ConvW cw = w.fh1;

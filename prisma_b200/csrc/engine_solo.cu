@@ -50,8 +50,6 @@ int SoloEngine::init(const std::string& vin, int dev) {
   exact_head = true;  // "<variant>-fast": the single-pass fp16 head of round 1 (not mask-id faithful, ~40 % faster per frame)
   if (v.size() > 5 && v.substr(v.size() - 5) == "-fast") { exact_head = false; v = v.substr(0, v.size() - 5); }
   if (v.size() > 6 && v.substr(v.size() - 6) == "-exact") { exact_backbone = true; v = v.substr(0, v.size() - 6); }
-  if (const char* e = getenv("PRISMA_SOLO_HEAD")) exact_head = std::string(e) != "fast";
-  if (const char* e = getenv("PRISMA_SOLO_BACKBONE")) exact_backbone = std::string(e) == "exact";
   if (!exact_head) exact_backbone = false;  // the fp32-class backbone feeds the fp32-class head
   variant = v;
   if (v == "r101") { const int l[4] = {3, 4, 23, 3}; std::copy(l, l + 4, layers); scale_long = 1333; scale_short = 800; }

@@ -33,7 +33,6 @@ __device__ __forceinline__ void cv_cubic_coeffs_f(float x, float* f) {  // cv::i
 // ~(4/step)^2 = 9 outputs), the output row is written coalesced
 __global__ void k_raft_resize(const uint8_t* __restrict__ img, int H, int W, uint8_t* __restrict__ out, int h, int w,
                               double step) {
-  pdl_prologue();
   const int ox = blockIdx.x * blockDim.x + threadIdx.x;
   const int oy = blockIdx.y;
   if (ox >= w) return;
@@ -64,7 +63,6 @@ __global__ void k_raft_resize(const uint8_t* __restrict__ img, int H, int W, uin
 
 __global__ void k_raft_pad_norm(const uint8_t* __restrict__ rs, int h, int w, float* __restrict__ chw, int hp, int wp,
                                 int pad_l, int pad_t) {
-  pdl_prologue();
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
   const int y = blockIdx.y;
   if (x >= wp) return;
@@ -80,10 +78,10 @@ int raft_preprocess(const uint8_t* img, int H, int W, int h, int w, double fx, c
                     cudaStream_t s) {
   const double step = 1.0 / fx;  // cv::resize with dsize empty: inv_scale_x = inv_scale_y = fx, sampling step 1 / fx
   dim3 block(128), grid(ceil_div(w, 128), h);
-  PRISMA_CUDA_OK(pdl_launch(k_raft_resize, dim3(grid), dim3(block), 0, s, img, H, W, resized, h, w, step));
+  k_raft_resize<<<grid, block, 0, s>>>(img, H, W, resized, h, w, step);
   const int hp = h + pad[2] + pad[3], wp = w + pad[0] + pad[1];
   dim3 grid2(ceil_div(wp, 128), hp);
-  PRISMA_CUDA_OK(pdl_launch(k_raft_pad_norm, dim3(grid2), dim3(block), 0, s, resized, h, w, chw, hp, wp, pad[0], pad[2]));
+  k_raft_pad_norm<<<grid2, block, 0, s>>>(resized, h, w, chw, hp, wp, pad[0], pad[2]);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -94,7 +92,6 @@ int raft_preprocess(const uint8_t* img, int H, int W, int h, int w, double fx, c
 __device__ __forceinline__ uint32_t f2ord_pos(float f) { return __float_as_uint(f); }  // distances are >= 0
 
 __global__ void k_flow_max(const float2* __restrict__ flow, long long n, uint32_t* __restrict__ mx) {
-  pdl_prologue();
   float hi = 0.f;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const float2 f = flow[i];
@@ -104,7 +101,7 @@ __global__ void k_flow_max(const float2* __restrict__ flow, long long n, uint32_
   if ((threadIdx.x & 31) == 0) atomicMax(mx, f2ord_pos(hi));
 }
 __global__ void k_zero_u32(uint32_t* p) {
-  pdl_prologue(); *p = 0u; }
+  *p = 0u; }
 
 __device__ __forceinline__ uint8_t polar_channel_u8(float h6f, double off, double rad, double one_minus_rad) {
   double v = fmod(__dadd_rn((double)h6f, off) , 6.0);
@@ -117,7 +114,6 @@ __device__ __forceinline__ uint8_t polar_channel_u8(float h6f, double off, doubl
 
 __global__ void k_flow_encode(const float2* __restrict__ flow, long long n, const uint32_t* __restrict__ mx,
                               uint8_t* __restrict__ rgb, float* __restrict__ max_out) {
-  pdl_prologue();
   const float maxd = __uint_as_float(*mx);
   if (blockIdx.x == 0 && threadIdx.x == 0 && max_out) *max_out = maxd;
   const float PI_F = 3.14159274101257324f;  // float32(np.pi)
@@ -141,9 +137,9 @@ __global__ void k_flow_encode(const float2* __restrict__ flow, long long n, cons
 int flow_encode(const float* flow, int H, int W, uint8_t* rgb, uint32_t* mm_scratch, float* max_out, int num_sms,
                 cudaStream_t s) {
   const long long n = (long long)H * W;
-  PRISMA_CUDA_OK(pdl_launch(k_zero_u32, dim3(1), dim3(1), 0, s, mm_scratch));
-  PRISMA_CUDA_OK(pdl_launch(k_flow_max, dim3(num_sms * 4), dim3(256), 0, s, reinterpret_cast<const float2*>(flow), n, mm_scratch));
-  PRISMA_CUDA_OK(pdl_launch(k_flow_encode, dim3(num_sms * 8), dim3(256), 0, s, reinterpret_cast<const float2*>(flow), n, mm_scratch, rgb, max_out));
+  k_zero_u32<<<1, 1, 0, s>>>(mm_scratch);
+  k_flow_max<<<num_sms * 4, 256, 0, s>>>(reinterpret_cast<const float2*>(flow), n, mm_scratch);
+  k_flow_encode<<<num_sms * 8, 256, 0, s>>>(reinterpret_cast<const float2*>(flow), n, mm_scratch, rgb, max_out);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -172,7 +168,6 @@ __device__ __forceinline__ float norm2_f32(float x, float y) { return __fsqrt_rn
 // mask[i] = |f + warp(g, f)| < a1 * (|f| + |warp(g, f)|) + a2     (f = this direction's flow, g = the other one's)
 __global__ void k_consistency_mask(const float2* __restrict__ f, const float2* __restrict__ g, int H, int W, float a1,
                                    float a2, uint8_t* __restrict__ mask) {
-  pdl_prologue();
   const long long total = (long long)H * W;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int y = (int)(i / W), x = (int)(i - (long long)y * W);
@@ -185,17 +180,16 @@ __global__ void k_consistency_mask(const float2* __restrict__ f, const float2* _
 }
 int flow_consistency_masks(const float* fwd, const float* bwd, int H, int W, uint8_t* fwd_mask, uint8_t* bwd_mask,
                            int num_sms, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_consistency_mask, dim3(num_sms * 8), dim3(256), 0, s, reinterpret_cast<const float2*>(fwd), reinterpret_cast<const float2*>(bwd),
-                                                 H, W, 0.05f, 0.5f, fwd_mask));
-  PRISMA_CUDA_OK(pdl_launch(k_consistency_mask, dim3(num_sms * 8), dim3(256), 0, s, reinterpret_cast<const float2*>(bwd), reinterpret_cast<const float2*>(fwd),
-                                                 H, W, 0.05f, 0.5f, bwd_mask));
+  k_consistency_mask<<<num_sms * 8, 256, 0, s>>>(reinterpret_cast<const float2*>(fwd), reinterpret_cast<const float2*>(bwd),
+                                                 H, W, 0.05f, 0.5f, fwd_mask);
+  k_consistency_mask<<<num_sms * 8, 256, 0, s>>>(reinterpret_cast<const float2*>(bwd), reinterpret_cast<const float2*>(fwd),
+                                                 H, W, 0.05f, 0.5f, bwd_mask);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
 // encode_flow: u16 (2^15 + 256 f) per component + validity channel
 __global__ void k_flow_u16(const float2* __restrict__ f, const uint8_t* __restrict__ mask, long long n,
                            uint16_t* __restrict__ out) {
-  pdl_prologue();
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const float fx = __fadd_rn(32768.f, __fmul_rn(f[i].x, 256.f)), fy = __fadd_rn(32768.f, __fmul_rn(f[i].y, 256.f));
     const bool ok = mask[i] && fmaxf(fx, fy) < 65535.f && 0.f < fminf(fx, fy);
@@ -205,7 +199,7 @@ __global__ void k_flow_u16(const float2* __restrict__ f, const uint8_t* __restri
   }
 }
 int flow_encode_u16(const float* flow, const uint8_t* mask, int H, int W, uint16_t* out, int num_sms, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_flow_u16, dim3(num_sms * 8), dim3(256), 0, s, reinterpret_cast<const float2*>(flow), mask, (long long)H * W, out));
+  k_flow_u16<<<num_sms * 8, 256, 0, s>>>(reinterpret_cast<const float2*>(flow), mask, (long long)H * W, out);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -214,23 +208,22 @@ int flow_encode_u16(const float* flow, const uint8_t* mask, int H, int W, uint16
 // K14 (by linearity): avg_pool2d of the correlation volume over its last two dims == correlation with the
 // average-pooled fmap2.  Pool fmap2 (fp16 [P][C]) into the three coarser levels (floor sizes, corr.py:24-27).
 // ------------------------------------------------------------------------------------------------
-// The pooled features are fp16 like the features themselves (one K-slab).  PRISMA_CORR_POOL_LO=1 keeps them as an fp16
-// hi/lo pair ([hi(C) | lo(C)] per row, two K-slabs of the same GEMM: no rounding of the means at all) -- the round-2 default
-// until the oracle study (fp16 features, means rounded or not, 12 iterations) put the difference at 5e-6 of the largest
-// displacement against a 1e-3 budget, while the second slab made the coarse GEMM operand-bound (K = 512 for 128 KB of output).
+// The pooled features are fp16 like the features themselves (one K-slab).  An fp16 hi/lo pair of the means (two K-slabs: no
+// rounding of the means at all) was measured against it: the oracle study (fp16 features, means rounded or not, 12 iterations)
+// put the difference at 5e-6 of the largest displacement against a 1e-3 budget, while the second slab made the coarse GEMM
+// operand-bound (K = 512 for 128 KB of output).
 // One launch pools `frames` feature maps to all three coarse levels: grid.x = cells of level 3, then 2, then 1 (the 8 x 8
 // windows, the longest blocks, start first), grid.y = frame.  A thread owns two channels (half2 loads); the sum runs in
-// fp32 in raster order of the window, as before.  Level l lands at row coff[l] of the frame's [n123][2 C] operand.
+// fp32 in raster order of the window.  Level l lands at row coff[l] of the frame's [n123][C] operand.
 __global__ void k_pool_fmap(const __half* __restrict__ feat, size_t frame_stride, int W8, int C, __half* __restrict__ out,
-                            size_t out_frame_stride, PoolGeom g, int with_lo) {
-  pdl_prologue();
+                            size_t out_frame_stride, PoolGeom g) {
   int cell = blockIdx.x, lvl = 3;
   if (cell >= g.ln[3]) { cell -= g.ln[3]; lvl = 2; if (cell >= g.ln[2]) { cell -= g.ln[2]; lvl = 1; } }
   const int lw = g.lw[lvl], win = 1 << lvl;
   const int y = cell / lw, x = cell - y * lw;
   const float inv = 1.0f / (float)(win * win);
   const __half* f = feat + blockIdx.y * frame_stride;
-  __half* o = out + blockIdx.y * out_frame_stride + (size_t)(g.coff[lvl] + cell) * (with_lo ? 2 : 1) * C;
+  __half* o = out + blockIdx.y * out_frame_stride + (size_t)(g.coff[lvl] + cell) * C;
   for (int c = 2 * threadIdx.x; c < C; c += 2 * blockDim.x) {
     float a0 = 0.f, a1 = 0.f;
     for (int dy = 0; dy < win; ++dy) {
@@ -241,11 +234,7 @@ __global__ void k_pool_fmap(const __half* __restrict__ feat, size_t frame_stride
         a0 += v.x; a1 += v.y;
       }
     }
-    const float m0 = a0 * inv, m1 = a1 * inv;
-    const __half h0 = __float2half_rn(m0), h1 = __float2half_rn(m1);
-    *reinterpret_cast<__half2*>(o + c) = __halves2half2(h0, h1);
-    if (with_lo)
-      *reinterpret_cast<__half2*>(o + C + c) = __halves2half2(__float2half_rn(m0 - __half2float(h0)), __float2half_rn(m1 - __half2float(h1)));
+    *reinterpret_cast<__half2*>(o + c) = __halves2half2(__float2half_rn(a0 * inv), __float2half_rn(a1 * inv));
   }
 }
 
@@ -261,7 +250,6 @@ __global__ void k_corr_lookup(const float* __restrict__ v0, const float* __restr
                               int lh1, int lw1, int lp1, int lh2, int lw2, int lp2, int lh3, int lw3, int lp3,
                               const float* __restrict__ coords, __half* __restrict__ out, int out_ld, int out_wp,
                               int out_pad, int out_img_rows) {
-  pdl_prologue();
   const int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (wid >= B * P) return;
@@ -340,7 +328,7 @@ int FlowCorr::init(int dev, int batch, int h8, int w8, int n_frames, const int* 
   rows_pad = round_up(P, 256);
   PRISMA_TRY(fc_alloc(allocs, &feat, (size_t)NF * rows_pad * C));
   // Levels 1..3 share one operand buffer and one volume: the pooled features of a frame are the rows [coff[l], coff[l] + ln[l])
-  // of a [n123][2 C] matrix, so ONE GEMM per direction writes the three coarse levels side by side into rows of pitch
+  // of a [n123][C] matrix, so ONE GEMM per direction writes the three coarse levels side by side into rows of pitch
   // pitch123 (level l = columns coff[l]...).  Two launches per direction instead of four: the coarse levels used to run
   // at 2.8-3.7 TB/s against level 0's 5.1 (short launches, 8-wave ramp each).
   coff[0] = 0;
@@ -353,15 +341,13 @@ int FlowCorr::init(int dev, int batch, int h8, int w8, int n_frames, const int* 
   rows123_pad = round_up(pitch123, 256);
   lpitch[0] = round_up(ln[0], 4);
   lrows_pad[0] = rows_pad;
-  pool_lo = [] { const char* e = getenv("PRISMA_CORR_POOL_LO"); return e && e[0] == '1'; }();
-  pw = pool_lo ? 2 : 1;
-  PRISMA_TRY(fc_alloc(allocs, &pool123, (size_t)NF * rows123_pad * C * pw));
+  PRISMA_TRY(fc_alloc(allocs, &pool123, (size_t)NF * rows123_pad * C));
   PRISMA_TRY(fc_alloc(allocs, &vol[0], (size_t)B * P * lpitch[0]));
   PRISMA_TRY(fc_alloc(allocs, &vol123, (size_t)B * P * pitch123));
   for (int l = 1; l < 4; ++l) {
     lpitch[l] = pitch123;
     lrows_pad[l] = rows123_pad;
-    pool[l] = pool123 + (size_t)coff[l] * C * pw;
+    pool[l] = pool123 + (size_t)coff[l] * C;
     vol[l] = vol123 + coff[l];
   }
   PRISMA_TRY(fc_alloc(allocs, &coords, (size_t)B * 2 * P));
@@ -377,12 +363,10 @@ int FlowCorr::init(int dev, int batch, int h8, int w8, int n_frames, const int* 
       ep.out_f32 = part == 0 ? vol[0] + (size_t)b * P * lpitch[0] : vol123 + (size_t)b * P * pitch123;
       ep.out_f32_ld = ncols;
       // the volume is store-bound (131 KB per 128 x 256 tile against 4 K-blocks of MMA): leave through TMA bulk stores
-      static const bool tma_off = [] { const char* e = getenv("PRISMA_CORR_TMA_STORE"); return e && e[0] == '0'; }();
       GemmLaunch g;
-      ep.tma_store = !tma_off && gemm_pick_bn(P, ncols, num_sms) >= 128;
-      const int wk = part == 0 ? 1 : pw;  // PRISMA_CORR_POOL_LO: against [hi | lo] pooled features = two K-slabs
-      const __half* w2 = part == 0 ? feat + (size_t)f2[b] * rows_pad * C : pool123 + (size_t)f2[b] * rows123_pad * C * pw;
-      PRISMA_TRY(gemm_prepare(&g, feat + (size_t)f1[b] * rows_pad * C, P, C, C, w2, part == 0 ? rows_pad : rows123_pad, P, ncols, wk,
+      ep.tma_store = gemm_pick_bn(P, ncols, num_sms) >= 128;
+      const __half* w2 = part == 0 ? feat + (size_t)f2[b] * rows_pad * C : pool123 + (size_t)f2[b] * rows123_pad * C;
+      PRISMA_TRY(gemm_prepare(&g, feat + (size_t)f1[b] * rows_pad * C, P, C, C, w2, part == 0 ? rows_pad : rows123_pad, P, ncols, 1,
                               off, ep, num_sms));
       gemms.push_back(g);
     }
@@ -413,9 +397,10 @@ int FlowCorr::set_fmaps(const float* fm1, const float* fm2) {
 int FlowCorr::pool_frames(int first, int count, cudaStream_t s) {
   PoolGeom g;
   for (int l = 0; l < 4; ++l) { g.lh[l] = lh[l]; g.lw[l] = lw[l]; g.ln[l] = ln[l]; g.coff[l] = coff[l]; }
-  PRISMA_CUDA_OK(pdl_launch(k_pool_fmap, dim3(ln[1] + ln[2] + ln[3], count), dim3(128), 0, s, (const __half*)(feat + (size_t)first * rows_pad * C),
-                            (size_t)rows_pad * C, W8, C, pool123 + (size_t)first * rows123_pad * C * pw, (size_t)rows123_pad * C * pw, g,
-                            pool_lo ? 1 : 0));
+  k_pool_fmap<<<dim3(ln[1] + ln[2] + ln[3], count), 128, 0, s>>>((const __half*)(feat + (size_t)first * rows_pad * C),
+                                                                 (size_t)rows_pad * C, W8, C, pool123 + (size_t)first * rows123_pad * C,
+                                                                 (size_t)rows123_pad * C, g);
+  PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
@@ -436,10 +421,10 @@ int FlowCorr::lookup(const float* d_coords, cudaStream_t s) {
 int FlowCorr::lookup_to(const float* d_coords, __half* dst, int dst_ld, int dst_wp, int dst_pad, int dst_img_rows,
                         cudaStream_t s) {
   const int warps = B * P;
-  PRISMA_CUDA_OK(pdl_launch(k_corr_lookup, dim3(ceil_div(warps * 32, 256)), dim3(256), 0, s, vol[0], vol[1], vol[2], vol[3], B, P, H8, W8, lh[0], lw[0],
+  k_corr_lookup<<<ceil_div(warps * 32, 256), 256, 0, s>>>(vol[0], vol[1], vol[2], vol[3], B, P, H8, W8, lh[0], lw[0],
                                                           lpitch[0], lh[1], lw[1], lpitch[1], lh[2], lw[2], lpitch[2],
                                                           lh[3], lw[3], lpitch[3], d_coords, dst, dst_ld, dst_wp,
-                                                          dst_pad, dst_img_rows));
+                                                          dst_pad, dst_img_rows);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -41,10 +41,8 @@ class FlowCorr {
   int NF = 0;                          // frames held
   int f1[8] = {0}, f2[8] = {0};        // frame of image1 / image2 per direction
   __half* feat = nullptr;              // [NF][rows_pad][C] fp16 features (rows padded to the next multiple of 256)
-  // levels 1..3 of a frame: rows [coff[l], coff[l] + ln[l]) of pool123 [NF][rows123_pad][pw C] = the 2^l x 2^l mean (fp16; pw = 2:
-  // [hi | lo]); pool[l] / vol[l] point at level l inside the shared buffers (rows123_pad * pw C per frame / pitch123 per position)
-  bool pool_lo = false;
-  int pw = 1;
+  // levels 1..3 of a frame: rows [coff[l], coff[l] + ln[l]) of pool123 [NF][rows123_pad][C] = the 2^l x 2^l mean (fp16);
+  // pool[l] / vol[l] point at level l inside the shared buffers (rows123_pad * C per frame / pitch123 per position)
   __half* pool123 = nullptr;
   float* vol123 = nullptr;
   int coff[4] = {0, 0, 0, 0}, n123 = 0, pitch123 = 0, rows123_pad = 0;

@@ -10,15 +10,6 @@ namespace prisma {
 NvtxRange::NvtxRange(const char* name) { nvtxRangePushA(name); }
 NvtxRange::~NvtxRange() { nvtxRangePop(); }
 
-// Programmatic dependent launch is OFF unless PRISMA_PDL=1.  Measured on B200 (bench.py, 1080p depth + flow): 86.3 frames/s
-// with it, 88.7 without -- the early-resident CTAs of the next kernel take issue slots from the running one and the ~330
-// kernels of a RAFT pass are already back to back inside a CUDA graph -- and tests/test_raft_gpu.py saw a wrong max
-// displacement under it (an ordering it must not change).  Kept only as an experiment switch.
-bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("PRISMA_PDL"); return e && e[0] == '1'; }();
-  return on;
-}
-
 static thread_local std::string g_last_error;
 void set_last_error(const std::string& msg) { g_last_error = msg; }
 const char* get_last_error() { return g_last_error.c_str(); }
@@ -130,15 +121,11 @@ int gemm_prepare_tf32x3(GemmLaunch* out, const float* A_split, long long a_rows,
   int off[GEMM_MAX_TAPS], acol[GEMM_MAX_TAPS];
   for (int t = 0; t < taps; ++t)
     for (int p = 0; p < 3; ++p) { off[t * 3 + p] = tap_off[t]; acol[t * 3 + p] = p == 1 ? C_half : 0; }
-  // external accumulation (GemmArgs::acc_group): 128-wide tiles at most (the running sums are 64 registers per thread), no
-  // narrow tail tiles.  PRISMA_TF32_ACC_GROUP=0 keeps the whole K inside one TMEM chain (the biased, cheaper variant).
-  static const int acc_group = [] { const char* e = getenv("PRISMA_TF32_ACC_GROUP"); return e ? atoi(e) : 4; }();
-  if (acc_group > 0 && force_bn == 0) force_bn = N > 64 ? 128 : (N > 32 ? 64 : 32);
-  PRISMA_TRY(gemm_prepare_impl(out, A_split, a_rows, C, 2 * C_half, W3, w_rows, M, N, taps * 3, off, acol, ep, num_sms, force_bn, true));
-  out->args.acc_group = acc_group > 0 ? acc_group : 1;
-  out->xacc = acc_group > 0 && out->bn <= 128;
-  if (out->xacc) { out->args.n_main = ceil_div(M, GEMM_BM) * ceil_div(N, out->bn); out->args.tail_split = 1; out->tmBt = out->tmB; }
-  return 0;
+  // external accumulation (GEMM_TF32_ACC_GROUP): 128-wide tiles at most (the running sums are 64 registers per thread), no
+  // narrow tail tiles
+  PRISMA_CHECK(force_bn <= 128, "gemm(tf32x3): BLOCK_N is at most 128");
+  if (force_bn == 0) force_bn = N > 64 ? 128 : (N > 32 ? 64 : 32);
+  return gemm_prepare_impl(out, A_split, a_rows, C, 2 * C_half, W3, w_rows, M, N, taps * 3, off, acol, ep, num_sms, force_bn, true);
 }
 
 static int gemm_prepare_impl(GemmLaunch* out, const void* A, long long a_rows, int a_cols, int a_pitch, const void* W,
@@ -148,38 +135,28 @@ static int gemm_prepare_impl(GemmLaunch* out, const void* A, long long a_rows, i
   PRISMA_CHECK(N % 4 == 0, "gemm: N must be a multiple of 4");
   PRISMA_CHECK(M >= 1 && a_cols >= 1, "gemm: empty problem");
   // force_bn == 512 requests the CTA-pair kernel (256 x 256 tiles); otherwise it is chosen for large problems
-  static const bool pairs_off = [] { const char* e = getenv("PRISMA_GEMM_PAIRS"); return e && e[0] == '0'; }();
   int bn = force_bn ? force_bn : gemm_pick_bn(M, N, num_sms);
   // the TMA-store epilogue exists for 128- and 256-wide tiles; a problem the tile choice gives narrower tiles keeps the
   // register epilogue (same results: the TMA path is an optimisation of the same arithmetic)
   GemmEpilogue ep = ep_in;
   if (ep.tma_store && (bn == 32 || bn == 64) && !tf32) ep.tma_store = false;
   int cg = 1;
-  static const bool pair128 = [] { const char* e = getenv("PRISMA_GEMM_PAIR128"); return e && e[0] == '1'; }();
   if (bn == 512) { bn = 256; cg = 2; }
-  else if (bn == 384) { bn = 128; cg = 2; }  // force: 256 x 128 CTA-pair tiles
-  else if (!force_bn && !pairs_off && !tf32 && bn == 256 && M >= 1024 && N >= 256) cg = 2;
-  else if (!force_bn && !pairs_off && !tf32 && pair128 && bn == 128 && M >= 4096 && N >= 128 && !ep.tma_store) cg = 2;
+  else if (!force_bn && !tf32 && bn == 256 && M >= 1024 && N >= 256) cg = 2;
   PRISMA_CHECK(!(tf32 && cg == 2), "gemm: the tf32 path has no CTA-pair instantiation");
   // Transposed tiles (GemmCfg SWAP) when one 128-wide tile covers all output columns: an M = 128 instruction costs the tensor
   // core >= 128 cycles whatever its N, so 128 x 256 (weights x rows) runs at twice the rate of 128 x 128 (rows x weights).
-  // PRISMA_GEMM_SWAP=0 switches it off; force_bn == 640 requests it.
-  static const bool swap_off = [] { const char* e = getenv("PRISMA_GEMM_SWAP"); return e && e[0] == '0'; }();
+  // force_bn == 640 requests it.
   bool swap = false;
   if (bn == 640) { bn = 128; cg = 1; swap = true; }
-  else if (!force_bn && !swap_off && !tf32 && cg == 1 && bn == 128 && N <= 128 && M >= 4096 && !ep.tma_store && !ep.head_w && !ep.m_dev) swap = true;
-  else {
-    // 64 output columns: the same transposed tile with the upper 64 weight rows zero (they must exist: w_rows >= 128) -- twice
-    // the MMA work of a 128 x 64 tile, but half the instructions, barriers and TMA boxes per output row (RAFT pass 6.73 -> 6.57 ms per pair).  PRISMA_GEMM_SWAP64=0: off.
-    static const bool swap64 = [] { const char* e = getenv("PRISMA_GEMM_SWAP64"); return !(e && e[0] == '0'); }();
-    if (swap64 && !force_bn && !swap_off && !tf32 && cg == 1 && bn == 64 && N > 32 && N <= 64 && w_rows >= 128 && M >= 4096 &&
-        !ep.tma_store && !ep.head_w && !ep.m_dev) { bn = 128; swap = true; }
-  }
+  else if (!force_bn && !tf32 && cg == 1 && bn == 128 && N <= 128 && M >= 4096 && !ep.tma_store && !ep.head_w && !ep.m_dev) swap = true;
+  // 64 output columns: the same transposed tile with the upper 64 weight rows zero (they must exist: w_rows >= 128) -- twice
+  // the MMA work of a 128 x 64 tile, but half the instructions, barriers and TMA boxes per output row (RAFT pass 6.73 -> 6.57 ms per pair)
+  else if (!force_bn && !tf32 && cg == 1 && bn == 64 && N > 32 && N <= 64 && w_rows >= 128 && M >= 4096 && !ep.tma_store &&
+           !ep.head_w && !ep.m_dev) { bn = 128; swap = true; }
   PRISMA_CHECK(!swap || (N <= 128 && !tf32 && !ep.tma_store && !ep.head_w), "gemm: transposed tiles need N <= 128, fp16 operands, the plain epilogue");
   out->swap = swap;
   out->tf32 = tf32;
-  out->xacc = false;
-  out->args.acc_group = 1;
   const int bke = tf32 ? 32 : 64;  // elements per 128-byte K block
   PRISMA_CHECK(bn == 32 || bn == 64 || bn == 128 || bn == 256, "gemm: unsupported BLOCK_N");
   PRISMA_CHECK(!swap || a_rows >= 1, "gemm: empty operand");
@@ -191,14 +168,7 @@ static int gemm_prepare_impl(GemmLaunch* out, const void* A, long long a_rows, i
   out->args.N = N;
   out->args.taps = taps;
   out->args.kchunks = kchunks;
-  {
-    static const char* r = getenv("PRISMA_GEMM_RASTER");  // "m" / "n": force (experiments)
-    out->args.raster_n = r ? (r[0] == 'n') : (M >= N);
-  }
-  {
-    static const int dbg = [] { const char* e = getenv("PRISMA_GEMM_DBG"); return e ? atoi(e) : 0; }();
-    out->args.dbg_mode = dbg;
-  }
+  out->args.raster_n = M >= N;
   for (int t = 0; t < GEMM_MAX_TAPS; ++t) {
     out->args.tap_off[t] = t < taps ? tap_off[t] : 0;
     out->args.tap_acol[t] = (t < taps && tap_acol) ? tap_acol[t] : 0;
@@ -222,10 +192,9 @@ static int gemm_prepare_impl(GemmLaunch* out, const void* A, long long a_rows, i
   out->args.tail_split = 1;
   out->tmBt = out->tmB;
   {
-    static const bool tail_off = [] { const char* e = getenv("PRISMA_GEMM_TAIL"); return e && e[0] == '0'; }();
     const int full = tiles / groups, rem = tiles % groups;
     auto cost = [](int w) { return w >= 256 ? 134.0 : (w >= 128 ? 100.0 : (w >= 64 ? 68.0 : 51.0)); };
-    if (!tail_off && !force_bn && !swap && full >= 1 && rem > 0) {
+    if (!force_bn && !swap && full >= 1 && rem > 0) {  // fp16 only: the 3xTF32 path always forces its tile width
       int best_split = 1;
       double best = cost(bn);
       for (int split = 2; split <= 4; split *= 2) {
@@ -237,10 +206,8 @@ static int gemm_prepare_impl(GemmLaunch* out, const void* A, long long a_rows, i
       if (best_split > 1) {
         out->args.n_main = full * groups;
         out->args.tail_split = best_split;
-        if (tf32) PRISMA_TRY(make_tmap_2d_f32(&out->tmBt, W, (uint64_t)taps * kchunks * 32, (uint64_t)w_rows,
-                                              (uint64_t)taps * kchunks * 32, 32, bn / best_split));
-        else PRISMA_TRY(make_tmap_2d_f16(&out->tmBt, W, (uint64_t)taps * kchunks * 64, (uint64_t)w_rows,
-                                         (uint64_t)taps * kchunks * 64, 64, bn / best_split / cg));
+        PRISMA_TRY(make_tmap_2d_f16(&out->tmBt, W, (uint64_t)taps * kchunks * 64, (uint64_t)w_rows,
+                                    (uint64_t)taps * kchunks * 64, 64, bn / best_split / cg));
       }
     }
   }
@@ -273,12 +240,12 @@ static int gemm_prepare_impl(GemmLaunch* out, const void* A, long long a_rows, i
   return 0;
 }
 
-template <int BN, int CG, bool TMAST = false, bool TF32 = false, bool XACC = false, bool SWAP = false, int EW = GEMM_EPI_WARPS>
+template <int BN, int CG, bool TMAST = false, bool TF32 = false, bool SWAP = false, int EW = GEMM_EPI_WARPS>
 static int launch_bn(const GemmLaunch& g, cudaStream_t stream) {
   static bool attr_set = false;  // per-process, per-instantiation
   using Cfg = GemmCfg<BN, CG, TMAST, SWAP, EW>;
   if (!attr_set) {
-    PRISMA_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<BN, CG, TMAST, TF32, XACC, SWAP, EW>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    PRISMA_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<BN, CG, TMAST, TF32, SWAP, EW>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
     attr_set = true;
   }
   {
@@ -287,39 +254,20 @@ static int launch_bn(const GemmLaunch& g, cudaStream_t stream) {
     cfg.blockDim = dim3(Cfg::THREADS);
     cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
     cfg.stream = stream;
-    cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (CG == 2) {
-      attr[na].id = cudaLaunchAttributeClusterDimension;
-      attr[na].val.clusterDim.x = CG; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
-      ++na;
-    }
-    if (pdl_enabled()) {  // the kernel waits (griddepcontrol.wait) after its prologue: safe after any predecessor
-      attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[na].val.programmaticStreamSerializationAllowed = 1;
-      ++na;
-    }
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = na;
-    PRISMA_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, CG, TMAST, TF32, XACC, SWAP, EW>, g.tmA, g.tmB, g.tmBt, g.tmD, g.args));
+    cfg.numAttrs = CG == 2 ? 1 : 0;
+    PRISMA_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, CG, TMAST, TF32, SWAP, EW>, g.tmA, g.tmB, g.tmBt, g.tmD, g.args));
   }
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
 int gemm_run(const GemmLaunch& g, cudaStream_t stream) {
-  if (g.tf32 && g.xacc) {
+  if (g.tf32) {  // external accumulation: BLOCK_N <= 128 (gemm_prepare_tf32x3)
     switch (g.bn) {
-      case 128: return launch_bn<128, 1, false, true, true>(g, stream);
-      case 64: return launch_bn<64, 1, false, true, true>(g, stream);
-      case 32: return launch_bn<32, 1, false, true, true>(g, stream);
-    }
-    set_last_error("gemm_run: external accumulation needs BLOCK_N <= 128");
-    return -1;
-  }
-  if (g.tf32) {
-    switch (g.bn) {
-      case 256: return launch_bn<256, 1, false, true>(g, stream);
       case 128: return launch_bn<128, 1, false, true>(g, stream);
       case 64: return launch_bn<64, 1, false, true>(g, stream);
       case 32: return launch_bn<32, 1, false, true>(g, stream);
@@ -327,38 +275,6 @@ int gemm_run(const GemmLaunch& g, cudaStream_t stream) {
     set_last_error("gemm_run: unsupported BLOCK_N (tf32)");
     return -1;
   }
-  // 16 epilogue warps for the plain fp16 kernels (GemmCfg EW).
-  // Measured (same box, whole bench step): 16 warps everywhere: RAFT convs 4.53 -> 4.34 ms per pair but DA linears 16.7 ->
-  // 17.4 ms per pass and head convs 7.05 -> 7.38 (the 256-wide tiles lose an operand stage and spill 270 bytes per thread at the
-  // 96 registers ptxas then allocates).  Default: 16 for the transposed / narrow tiles, 8 for the 256-wide ones;
-  // PRISMA_GEMM_EW=8 / 16 forces one value everywhere.
-  static const int ew_env = [] { const char* e = getenv("PRISMA_GEMM_EW"); return e ? atoi(e) : 0; }();
-  static const int ew_narrow = [] { const char* e = getenv("PRISMA_GEMM_EW_NARROW"); return e ? atoi(e) : 16; }();  // 8 / 12 / 16
-  static const int ew_wide = [] { const char* e = getenv("PRISMA_GEMM_EW_WIDE"); return e ? atoi(e) : 8; }();
-  const int ew = ew_env ? ew_env : ((g.swap || (g.cg == 1 && g.bn <= 128)) ? ew_narrow : ew_wide);
-  if (ew == 16 && !g.tma_store) {
-    if (g.swap) return launch_bn<128, 1, false, false, false, true, 16>(g, stream);
-    if (g.cg == 2 && g.bn == 256) return launch_bn<256, 2, false, false, false, false, 16>(g, stream);
-    if (g.cg == 1) {
-      switch (g.bn) {
-        case 256: return launch_bn<256, 1, false, false, false, false, 16>(g, stream);
-        case 128: return launch_bn<128, 1, false, false, false, false, 16>(g, stream);
-        case 64: return launch_bn<64, 1, false, false, false, false, 16>(g, stream);
-      }
-    }
-  }
-  if (ew == 12 && !g.tma_store) {
-    if (g.swap) return launch_bn<128, 1, false, false, false, true, 12>(g, stream);
-    if (g.cg == 2 && g.bn == 256) return launch_bn<256, 2, false, false, false, false, 12>(g, stream);
-    if (g.cg == 1) {
-      switch (g.bn) {
-        case 256: return launch_bn<256, 1, false, false, false, false, 12>(g, stream);
-        case 128: return launch_bn<128, 1, false, false, false, false, 12>(g, stream);
-        case 64: return launch_bn<64, 1, false, false, false, false, 12>(g, stream);
-      }
-    }
-  }
-  if (g.swap) return launch_bn<128, 1, false, false, false, true>(g, stream);
   if (g.tma_store) {
     if (g.cg == 2 && g.bn == 256) return launch_bn<256, 2, true>(g, stream);
     if (g.cg == 1 && g.bn == 256) return launch_bn<256, 1, true>(g, stream);
@@ -366,16 +282,20 @@ int gemm_run(const GemmLaunch& g, cudaStream_t stream) {
     set_last_error("gemm_run: no TMA-store instantiation for this tile shape");
     return -1;
   }
+  // 16 epilogue warps (GemmCfg EW) for the transposed and the 128- / 64-wide single-CTA tiles, 8 for the 256-wide and the
+  // 32-wide ones.  Measured (same box, whole bench step): 16 warps everywhere: RAFT convs 4.53 -> 4.34 ms per pair but DA
+  // linears 16.7 -> 17.4 ms per pass and head convs 7.05 -> 7.38 (the 256-wide tiles lose an operand stage and spill 270 bytes
+  // per thread at the 96 registers ptxas then allocates).
+  if (g.swap) return launch_bn<128, 1, false, false, true, 16>(g, stream);
   if (g.cg == 2) {
     if (g.bn == 256) return launch_bn<256, 2>(g, stream);
-    if (g.bn == 128) return launch_bn<128, 2>(g, stream);
-    set_last_error("gemm_run: CTA pairs need BLOCK_N 256 or 128");
+    set_last_error("gemm_run: CTA pairs need BLOCK_N 256");
     return -1;
   }
   switch (g.bn) {
     case 256: return launch_bn<256, 1>(g, stream);
-    case 128: return launch_bn<128, 1>(g, stream);
-    case 64: return launch_bn<64, 1>(g, stream);
+    case 128: return launch_bn<128, 1, false, false, false, 16>(g, stream);
+    case 64: return launch_bn<64, 1, false, false, false, 16>(g, stream);
     case 32: return launch_bn<32, 1>(g, stream);
   }
   set_last_error("gemm_run: unsupported BLOCK_N");

@@ -27,6 +27,7 @@ constexpr int GEMM_EPI_WARPS = 8;                          // two per TMEM lane 
 constexpr int GEMM_THREADS = 64 + 32 * GEMM_EPI_WARPS;      // + TMA producer warp + MMA warp
 constexpr int GEMM_SMEM_MAX = 232448;                       // 227 KB of dynamic shared memory per CTA
 constexpr int GEMM_MAX_TAPS = 49;
+constexpr int GEMM_TF32_ACC_GROUP = 4;  // 3xTF32: K blocks per TMEM chain before the external fp32 add (see the MMA issuer)
 
 enum RowMap : int {
   ROW_LINEAR = 0,   // dst row = m                                   (valid: m < M)
@@ -116,18 +117,13 @@ struct GemmArgs {
                                 // [hi | lo] activation halves: (hi, W_hi), (lo, W_hi), (hi, W_lo)
   int n_main;      // work items [0, n_main) are full BN-wide tiles; the remaining tiles are each cut into `tail_split`
   int tail_split;  // narrower tiles (BN / tail_split wide) so the last partial wave costs a fraction of a full one; 1 = off
-  int acc_group;  // XACC kernels: K blocks accumulated inside one TMEM chain before the partial sum is added to the running
-                  // fp32 sums held in the epilogue warps' registers (see gemm_prepare_tf32x3)
-  int dbg_mode;  // diagnostics (PRISMA_GEMM_DBG): 1 = prologue + teardown only, 2 = loads + MMAs but the epilogue warps only
-                 // release the accumulators, 3 = loads only (the MMA warp commits without issuing), 4 = taps one row after
-                 // the previous tap skip their A load, 5 = no loads (MMAs on whatever shared memory holds), 6 = 5 + no epilogue
   int raster_n;  // 1: consecutive tiles walk N first (the CTAs of a wave share few A row panels and all of W: A is read
                  // from HBM once when M >> N); 0: M first
   GemmEpilogue ep;
 };
 
 // SWAP ("swap A/B", BN == 128, CG == 1): the tensor core spends >= 128 cycles on every M = 128 instruction whatever its N
-// (measured, tools/gemm_pace.py: N = 128 tiles reach half the rate of N = 256 ones with no loads and no epilogue), so a
+// (measured: N = 128 tiles reach half the rate of N = 256 ones with no loads and no epilogue), so a
 // GEMM with <= 128 output columns runs transposed: the WEIGHT tile (128 output channels) is the M operand, 256 pixel rows
 // are the N operand of one instruction, the accumulator holds channels in its lanes and pixels in its columns, and the
 // epilogue transposes through its staging buffer (which it does anyway).  Half the instructions, barriers and TMA boxes
@@ -135,8 +131,7 @@ struct GemmArgs {
 // EW: epilogue warps (EW / 4 per TMEM lane quarter, taking every (EW / 4)-th 32-column chunk).  The epilogue is latency-bound
 // (ncu on fc1: issue slots 25 % busy, long-scoreboard / wait stalls) and paces the kernel (DESIGN 4.1), so the fp16 kernels can
 // run 16 of them: half the chunks per warp; one operand stage is given up for the staging buffers and the register cap
-// drops: 18 warps put 5 on one scheduler's 16 K registers = 96 per thread (spills 100-280 bytes), 14 warps (EW = 12) keep 128
-// (spills 40-64 bytes).
+// drops: 18 warps put 5 on one scheduler's 16 K registers = 96 per thread (spills 100-280 bytes).
 template <int BN, int CG = 1, bool TMAST = false, bool SWAP = false, int EW = GEMM_EPI_WARPS>  // CG = CTAs per MMA (cta_group): 2 = a CTA pair computes a 256 x BN tile, each loading half of W
 struct GemmCfg {                                   // TMAST: TMA-store epilogue (double-buffered staging, one operand stage fewer)
   static constexpr int A_ROWS = SWAP ? 256 : GEMM_BM;   // activation rows per tile and CTA
@@ -299,13 +294,14 @@ __device__ __forceinline__ void epilogue_rows8(const GemmEpilogue& ep, float4 (&
   }
 }
 
-template <int BN, int CG, bool TMAST, bool TF32, bool XACC, bool SWAP = false, int EW = GEMM_EPI_WARPS>
+template <int BN, int CG, bool TMAST, bool TF32, bool SWAP = false, int EW = GEMM_EPI_WARPS>
 __global__ void __launch_bounds__(64 + 32 * EW, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmBt, const __grid_constant__ CUtensorMap tmD,
                const __grid_constant__ GemmArgs args) {
-  static_assert(!SWAP || (BN == 128 && CG == 1 && !TMAST && !TF32 && !XACC), "SWAP: 128 output channels x 256 pixel rows, fp16, one CTA");
-  static_assert(EW == 8 || ((EW == 12 || EW == 16) && !TMAST && !TF32 && !XACC), "12 / 16 epilogue warps: the plain fp16 kernels only");
+  static_assert(!SWAP || (BN == 128 && CG == 1 && !TMAST && !TF32), "SWAP: 128 output channels x 256 pixel rows, fp16, one CTA");
+  static_assert(!TF32 || (BN <= 128 && CG == 1 && !TMAST), "TF32 (external accumulation): BN <= 128, one CTA, register epilogue");
+  static_assert(EW == 8 || (EW == 16 && !TMAST && !TF32), "16 epilogue warps: the plain fp16 kernels only");
   using Cfg = GemmCfg<BN, CG, TMAST, SWAP, EW>;
   constexpr int ACC = Cfg::ACC_COLS;
   constexpr int CSTEP = 32 * (EW / 4);  // column distance between the chunks one warp takes
@@ -326,7 +322,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   uint64_t* tempty = bars + 2 * STAGES + 2;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 4);
 
-  pdl_launch_dependents();  // the next kernel may be scheduled behind this one (see common.cuh)
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int rank = CG == 2 ? (int)cluster_ctarank() : 0;  // position inside the CTA pair
@@ -361,13 +356,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (CG == 2) cluster_sync_all(); else __syncthreads();  // the peer's barriers must exist before anything targets them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();  // barriers, TMEM and descriptors are set up; from here on the predecessor's results are read
 
-  if (args.dbg_mode == 1) {
-    // diagnostics: nothing but the prologue and the teardown
-  } else if (warp == 0) {
+  if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer
-    if (lane == 0 && args.dbg_mode != 5 && args.dbg_mode != 6) {  // dbg_mode 5 / 6: no operand loads at all (the MMA warp does not wait)
+    if (lane == 0) {
       int stage = 0; uint32_t phase = 0;
       for (int tile = group; tile < num_items; tile += num_groups) {
         int tm, tn, nsub, bw;
@@ -379,17 +371,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         int tap = 0, chunk = 0;
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(&empty[stage], phase ^ 1);
-          // diagnostics (dbg_mode 4): taps that shift the previous tap's rows by exactly one row do not load A at all (the
-          // MMAs read stale tiles; results are garbage) -- the upper bound of what a shared row-halo A tile would save
-          const bool skip_a = args.dbg_mode == 4 && tap > 0 && args.tap_off[tap] == args.tap_off[tap - 1] + 1;
           if (CG == 2) {
             // both CTAs' bytes land on the leader's barrier; only the leader arrives (count 1) and posts the total
-            if (rank == 0) mbar_arrive_expect_tx(&full[stage], 2 * (stage_bytes - (skip_a ? Cfg::A_BYTES : 0)));
-            if (!skip_a) tma_load_2d_pair(sA + stage * Cfg::A_BYTES, &tmA, &full[stage], args.tap_acol[tap] + chunk * BKE, m0 + args.tap_off[tap]);
+            if (rank == 0) mbar_arrive_expect_tx(&full[stage], 2 * stage_bytes);
+            tma_load_2d_pair(sA + stage * Cfg::A_BYTES, &tmA, &full[stage], args.tap_acol[tap] + chunk * BKE, m0 + args.tap_off[tap]);
             tma_load_2d_pair(sB + stage * Cfg::B_BYTES, tb, &full[stage], kb * BKE, n0);
           } else {
-            mbar_arrive_expect_tx(&full[stage], stage_bytes - (skip_a ? Cfg::A_BYTES : 0));
-            if (!skip_a) tma_load_2d(sA + stage * Cfg::A_BYTES, &tmA, &full[stage], args.tap_acol[tap] + chunk * BKE, m0 + args.tap_off[tap]);
+            mbar_arrive_expect_tx(&full[stage], stage_bytes);
+            tma_load_2d(sA + stage * Cfg::A_BYTES, &tmA, &full[stage], args.tap_acol[tap] + chunk * BKE, m0 + args.tap_off[tap]);
             tma_load_2d(sB + stage * Cfg::B_BYTES, tb, &full[stage], kb * BKE, n0);
           }
           if (++chunk == args.kchunks) { chunk = 0; ++tap; }
@@ -401,15 +390,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // ------------------------------------------------------------------ MMA issuer (leader CTA of the pair only)
     if (lane == 0 && rank == 0) {
       constexpr uint32_t idesc_full = SWAP ? make_idesc_f16(128, 256) : (TF32 ? make_idesc_tf32(TILE_M, BN) : make_idesc_f16(TILE_M, BN));
-      const uint32_t idesc_tail = TF32 ? make_idesc_tf32(TILE_M, bw_tail) : make_idesc_f16(TILE_M, bw_tail);
+      const uint32_t idesc_tail = make_idesc_f16(TILE_M, bw_tail);
       int stage = 0; uint32_t phase = 0;
       int it = 0;
-      if (XACC) {
+      if (TF32) {
         // External accumulation: the tensor core adds into its fp32 accumulator by TRUNCATING the aligned addend, a bias
         // that grows with the length of the chain (measured: 5e-6 of sum |a||w| after ~900 MMAs).  Here a chain is only
-        // `acc_group` K blocks long; every finished partial sum is handed to the epilogue warps (tfull), which add it
+        // GEMM_TF32_ACC_GROUP K blocks long; every finished partial sum is handed to the epilogue warps (tfull), which add it
         // to register-resident running sums with round-to-nearest FADDs, and the TMEM stage is reused (tempty).
-        const int G = args.acc_group;
+        constexpr int G = GEMM_TF32_ACC_GROUP;
         int gi = 0;  // partial sums issued so far (TMEM stage = gi & 1)
         for (int tile = group; tile < num_items; tile += num_groups) {
           for (int kb = 0; kb < num_kb; ++kb) {
@@ -421,10 +410,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const uint64_t adesc = make_sdesc_sw128(smem_u32(sA + stage * Cfg::A_BYTES));
             const uint64_t bdesc = make_sdesc_sw128(smem_u32(sB + stage * Cfg::B_BYTES));
 #pragma unroll
-            for (int k = 0; k < GEMM_BK / 16; ++k) {
-              if (TF32) umma_tf32(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc_full, (kg | k) != 0 ? 1u : 0u);
-              else umma_f16(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc_full, (kg | k) != 0 ? 1u : 0u);
-            }
+            for (int k = 0; k < GEMM_BK / 16; ++k)  // K = 8 fp32 = 32 B: +2 in the (addr >> 4) field
+              umma_tf32(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc_full, (kg | k) != 0 ? 1u : 0u);
             umma_commit(&empty[stage]);
             if (++stage == STAGES) { stage = 0; phase ^= 1; }
             if (kg == G - 1 || kb == num_kb - 1) { umma_commit(&tfull[gi & 1]); ++gi; }
@@ -439,17 +426,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + as * ACC;
         for (int kb = 0; kb < num_kb; ++kb) {
-          if (args.dbg_mode != 5 && args.dbg_mode != 6) mbar_wait(&full[stage], phase);
+          mbar_wait(&full[stage], phase);
           tc_fence_after();
           // SWAP: the weight tile is the M operand, the 256 activation rows the N operand
           const uint64_t adesc = make_sdesc_sw128(smem_u32(SWAP ? sB + stage * Cfg::B_BYTES : sA + stage * Cfg::A_BYTES));
           const uint64_t bdesc = make_sdesc_sw128(smem_u32(SWAP ? sA + stage * Cfg::A_BYTES : sB + stage * Cfg::B_BYTES));
 #pragma unroll
           for (int k = 0; k < GEMM_BK / 16; ++k) {
-            if (args.dbg_mode == 3) break;
             // advance 16 fp16 = 32 B along K inside the 128 B swizzled row: +2 in the (addr >> 4) field
-            if (TF32) umma_tf32(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);  // K = 8 fp32 = 32 B
-            else if (CG == 2) umma_f16_pair(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
+            if (CG == 2) umma_f16_pair(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
             else umma_f16(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
           }
           if (CG == 2) umma_commit_pair(&empty[stage]); else umma_commit(&empty[stage]);
@@ -468,7 +453,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int cg = lane & 7;     // coalesced phase: which 4-column group of the 32-column chunk
     const int rsub = lane >> 3;  // coalesced phase: row offset inside a 4-row step
     int it = 0;
-    int xgi = 0;  // XACC: partial sums consumed so far
+    int xgi = 0;  // TF32: partial sums consumed so far
     for (int tile = group; tile < num_items; tile += num_groups, ++it) {
       const int as = it & 1;
       const uint32_t aphase = (it >> 1) & 1;
@@ -640,9 +625,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
           for (int rr = 0; rr < 8; ++rr)
             drs[rr] = ib8[rr] + (ty8[rr] * ep.shuf_s + sdy + out_ld) * ep.out_wp + tx8[rr] * ep.shuf_s + sdx + out_ld;
-          epilogue_rows8<!TF32 && !XACC && !TMAST>(ep, v, drs, ncol_ok ? okrows : 0u, bias4, gamma4, col);
+          epilogue_rows8<!TF32 && !TMAST>(ep, v, drs, ncol_ok ? okrows : 0u, bias4, gamma4, col);
         } else {
-          epilogue_rows8<!TF32 && !XACC && !TMAST>(ep, v, dr8, ncol_ok ? okrows : 0u, bias4, gamma4, col);
+          epilogue_rows8<!TF32 && !TMAST>(ep, v, dr8, ncol_ok ? okrows : 0u, bias4, gamma4, col);
         }
         if (ep.stat_part != nullptr) {
           float4 sm = make_float4(0.f, 0.f, 0.f, 0.f), sq = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -668,15 +653,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         }
       
       };
-      if (XACC) {
-        // running sums of this warp's chunks live in registers; partial sums arrive every `acc_group` K blocks
+      if (TF32) {
+        // running sums of this warp's chunks live in registers; partial sums arrive every GEMM_TF32_ACC_GROUP K blocks
         constexpr int NCH = (BN + 63) / 64;
         float acc[NCH][32];
 #pragma unroll
         for (int i = 0; i < NCH; ++i)
 #pragma unroll
           for (int j = 0; j < 32; ++j) acc[i][j] = 0.f;
-        const int ngroups = (num_kb + args.acc_group - 1) / args.acc_group;
+        const int ngroups = (num_kb + GEMM_TF32_ACC_GROUP - 1) / GEMM_TF32_ACC_GROUP;
         for (int g = 0; g < ngroups; ++g, ++xgi) {
           const int xs = xgi & 1;
           mbar_wait(&tfull[xs], (xgi >> 1) & 1);
@@ -718,7 +703,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         // this warp: output columns n0 + quarter * 32 .. + 31 (TMEM lanes), alternate 32-pixel chunks (TMEM columns)
 #pragma unroll 1
         for (int c0 = chunk_par * 32; c0 < 256; c0 += CSTEP) {
-          if (m0 + c0 >= args.M || n0 + quarter * 32 >= args.N || args.dbg_mode == 2 || args.dbg_mode == 3 || args.dbg_mode == 6) break;  // warp-uniform
+          if (m0 + c0 >= args.M || n0 + quarter * 32 >= args.N) break;  // warp-uniform
           uint32_t r[32];
           tmem_ld32(taddr + c0, r);
           map_rows(m0 + c0);
@@ -732,7 +717,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         // 32 x 128-byte box, the same staging layout and swizzle as the fp32 path
 #pragma unroll 1
         for (int cb = chunk_par * 64; cb < bw; cb += 128) {
-          if (n0 + cb >= args.N || args.dbg_mode == 2 || args.dbg_mode == 3 || args.dbg_mode == 6) break;  // warp-uniform
+          if (n0 + cb >= args.N) break;  // warp-uniform
           const uint32_t buf = stg + (st_cnt & 1) * 4096;
           if (st_cnt >= 2) { if (lane == 0) tma_store_wait_read<1>(); __syncwarp(); }
 #pragma unroll
@@ -782,7 +767,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       } else
 #pragma unroll 1
       for (int c0 = chunk_par * 32; c0 < bw; c0 += CSTEP) {
-        if (n0 + c0 >= args.N || args.dbg_mode == 2 || args.dbg_mode == 3 || args.dbg_mode == 6) break;  // warp-uniform
+        if (n0 + c0 >= args.N) break;  // warp-uniform
         uint32_t r[32];
         tmem_ld32(taddr + c0, r);
         float4 bias4, gamma4;
@@ -811,8 +796,8 @@ struct GemmLaunch {
   CUtensorMap tmA, tmB, tmBt;  // tmBt: W with the narrow box of the tail tiles (== tmB when there is no tail)
   CUtensorMap tmD;             // dense output, 32 x 32 boxes (TMA-store epilogue only)
   bool tma_store = false;
-  bool xacc = false;           // external fp32 accumulation (tf32x3 only): see GemmArgs::acc_group
-  bool tf32 = false;           // kind::tf32 operands (fp32 containers): the 3xTF32 "fp32-class" path of the mask band
+  bool tf32 = false;           // kind::tf32 operands (fp32 containers): the 3xTF32 "fp32-class" path of the mask band, with
+                               // external fp32 accumulation (GEMM_TF32_ACC_GROUP)
   bool swap = false;           // transposed tiles for N <= 128: 128 output columns x 256 rows per instruction (GemmCfg SWAP)
   GemmArgs args;
   int bn = 128;

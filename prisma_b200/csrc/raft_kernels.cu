@@ -13,7 +13,6 @@ namespace prisma {
 // Stride 2 is applied here, no wasted rows.
 // ------------------------------------------------------------------------------------------------
 __global__ void k_im2col_stem(const float* __restrict__ x, int B, int H, int W, __half* __restrict__ out) {
-  pdl_prologue();
   // one thread = one (c, ky) row of one output pixel: 7 consecutive input floats -> a 16-byte store; consecutive threads =
   // consecutive groups, so a warp writes 512 contiguous bytes and its gathers walk the same few image rows
   const int Ho = H / 2, Wo = W / 2;
@@ -44,7 +43,7 @@ __global__ void k_im2col_stem(const float* __restrict__ x, int B, int H, int W, 
   }
 }
 int raft_im2col_stem(const float* x, int B, int H, int W, __half* out, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_im2col_stem, dim3(148 * 16), dim3(256), 0, s, x, B, H, W, out));
+  k_im2col_stem<<<148 * 16, 256, 0, s>>>(x, B, H, W, out);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -55,7 +54,6 @@ int raft_im2col_stem(const float* x, int B, int H, int W, __half* out, cudaStrea
 // a zero-bordered NHWC fp16 map.
 // ------------------------------------------------------------------------------------------------
 __global__ void k_in_partial(const float* __restrict__ x, int HW, int C, int rows_per_block, float* __restrict__ part) {
-  pdl_prologue();
   extern __shared__ float sh[];  // [groups][C][2]
   const int b = blockIdx.y, blk = blockIdx.x;
   const int groups = blockDim.x / C;
@@ -82,7 +80,6 @@ __global__ void k_in_partial(const float* __restrict__ x, int HW, int C, int row
   }
 }
 __global__ void k_in_final(const float* __restrict__ part, int nblk, int C, int HW, float eps, float* __restrict__ stats) {
-  pdl_prologue();
   // blockDim.x / C groups of C threads add interleaved stripes of the partial blocks in double, then group 0 adds the groups
   // (fixed order: deterministic)
   __shared__ double shd[512 * 2];
@@ -112,8 +109,8 @@ int instnorm_stats(const float* x, int B, int HW, int C, float* part, float* sta
   const int threads = C <= 64 ? 4 * C : 2 * C;
   const int rows_per_block = 512;
   const int nblk = ceil_div(HW, rows_per_block);
-  PRISMA_CUDA_OK(pdl_launch(k_in_partial, dim3(dim3(nblk, B)), dim3(threads), threads * 2 * sizeof(float), s, x, HW, C, rows_per_block, part));
-  PRISMA_CUDA_OK(pdl_launch(k_in_final, dim3(B), dim3(512), 0, s, part, nblk, C, HW, 1e-5f, stats));
+  k_in_partial<<<dim3(nblk, B), threads, threads * 2 * sizeof(float), s>>>(x, HW, C, rows_per_block, part);
+  k_in_final<<<B, 512, 0, s>>>(part, nblk, C, HW, 1e-5f, stats);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -121,7 +118,6 @@ int instnorm_stats(const float* x, int B, int HW, int C, float* part, float* sta
 // [b * spi, (b + 1) * spi).  Stage 1: nblk blocks per image add stripes of slabs in double (fixed order); stage 2: one
 // block per image adds the nblk partial sums and writes (mean, 1 / sqrt(var + eps)).  HW = number of pixels normalised.
 __global__ void k_in_slab_stage1(const float* __restrict__ part, int spi, int C, double* __restrict__ part2) {
-  pdl_prologue();
   extern __shared__ double shd[];  // [groups][C][2]
   const int b = blockIdx.y, blk = blockIdx.x, nblk = gridDim.x;
   const int groups = blockDim.x / C;
@@ -147,7 +143,6 @@ __global__ void k_in_slab_stage1(const float* __restrict__ part, int spi, int C,
   }
 }
 __global__ void k_in_slab_stage2(const double* __restrict__ part2, int nblk, int C, int HW, float eps, float* __restrict__ stats) {
-  pdl_prologue();
   const int b = blockIdx.x, c = threadIdx.x;
   if (c >= C) return;
   double s = 0.0, q = 0.0;
@@ -164,8 +159,8 @@ __global__ void k_in_slab_stage2(const double* __restrict__ part2, int nblk, int
 int instnorm_stats_from_slabs(const float* slab_part, int B, int slabs_per_image, int C, int HW, double* part2, float* stats,
                               cudaStream_t s) {
   const int threads = C <= 64 ? 4 * C : 2 * C, nblk = INSTNORM_STAGE1_BLOCKS;
-  PRISMA_CUDA_OK(pdl_launch(k_in_slab_stage1, dim3(dim3(nblk, B)), dim3(threads), threads * 2 * sizeof(double), s, slab_part, slabs_per_image, C, part2));
-  PRISMA_CUDA_OK(pdl_launch(k_in_slab_stage2, dim3(B), dim3(128), 0, s, part2, nblk, C, HW, 1e-5f, stats));
+  k_in_slab_stage1<<<dim3(nblk, B), threads, threads * 2 * sizeof(double), s>>>(slab_part, slabs_per_image, C, part2);
+  k_in_slab_stage2<<<B, 128, 0, s>>>(part2, nblk, C, HW, 1e-5f, stats);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -175,7 +170,6 @@ int instnorm_partial_floats(int B, int HW, int C) { return B * ceil_div(HW, 512)
 __global__ void k_in_apply(const float* __restrict__ x, const float* __restrict__ stats, int H, int W, int C,
                            const __half* __restrict__ skip_map, const float* __restrict__ skip_raw,
                            const float* __restrict__ skip_stats, __half* __restrict__ out, int pad, long long img_rows) {
-  pdl_prologue();
   const int c4 = C >> 2;
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long per_img = (long long)H * W * c4;
@@ -206,8 +200,8 @@ __global__ void k_in_apply(const float* __restrict__ x, const float* __restrict_
 int instnorm_apply(const float* x, const float* stats, int B, int H, int W, int C, const __half* skip_map,
                    const float* skip_raw, const float* skip_stats, __half* out, int pad, long long img_rows, cudaStream_t s) {
   const long long per_img = (long long)H * W * (C / 4);
-  PRISMA_CUDA_OK(pdl_launch(k_in_apply, dim3(dim3((unsigned)((per_img + 255) / 256), B)), dim3(256), 0, s, x, stats, H, W, C, skip_map, skip_raw, skip_stats,
-                                                                       out, pad, img_rows));
+  k_in_apply<<<dim3((unsigned)((per_img + 255) / 256), B), 256, 0, s>>>(x, stats, H, W, C, skip_map, skip_raw, skip_stats,
+                                                                        out, pad, img_rows);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -219,7 +213,6 @@ int instnorm_apply(const float* x, const float* stats, int B, int H, int W, int 
 // cn holds the context features per FRAME; direction b reads those of frame df.f[b] (its image1).
 __global__ void k_cnet_split(const float* __restrict__ cn, int B, int H, int W, int pad, long long img_rows, DirFrames df,
                              float* __restrict__ h_master, __half* __restrict__ hx, __half* __restrict__ rhx) {
-  pdl_prologue();
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // over B*H*W*256
   const long long total = (long long)B * H * W * 256;
   if (idx >= total) return;
@@ -244,7 +237,7 @@ __global__ void k_cnet_split(const float* __restrict__ cn, int B, int H, int W, 
 int raft_cnet_split(const float* cn, int B, int H, int W, int pad, long long img_rows, DirFrames df, float* h_master, __half* hx,
                     __half* rhx, cudaStream_t s) {
   const long long total = (long long)B * H * W * 256;
-  PRISMA_CUDA_OK(pdl_launch(k_cnet_split, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, cn, B, H, W, pad, img_rows, df, h_master, hx, rhx));
+  k_cnet_split<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(cn, B, H, W, pad, img_rows, df, h_master, hx, rhx);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -255,7 +248,6 @@ int raft_cnet_split(const float* cn, int B, int H, int W, int pad, long long img
 // a single fp16 would cost 8e-4 of the 1e-3 budget).  Row = pixel, K = [98 hi | 30 zero | 98 lo | 30 zero].
 __global__ void k_flow_im2col(const float* __restrict__ coords0, const float* __restrict__ coords1, int B, int H, int W,
                               __half* __restrict__ out) {
-  pdl_prologue();
   // one thread = 8 consecutive k of one pixel: two 16-byte stores (hi and lo halves); a warp covers two whole rows
   const int P = H * W;
   const long long total = (long long)B * P * 16;
@@ -290,7 +282,7 @@ __global__ void k_flow_im2col(const float* __restrict__ coords0, const float* __
   }
 }
 int raft_flow_im2col(const float* coords0, const float* coords1, int B, int H, int W, __half* out, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_flow_im2col, dim3(148 * 8), dim3(256), 0, s, coords0, coords1, B, H, W, out));
+  k_flow_im2col<<<148 * 8, 256, 0, s>>>(coords0, coords1, B, H, W, out);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -298,7 +290,6 @@ int raft_flow_im2col(const float* coords0, const float* coords1, int B, int H, i
 // motion features = cat([conv_out(126), flow(2)]) (update.py:97): the two flow channels of the GRU operand maps
 __global__ void k_flow_cols(const float* __restrict__ c0, const float* __restrict__ c1, int B, int H, int W, int pad,
                             long long img_rows, __half* __restrict__ hx, __half* __restrict__ rhx) {
-  pdl_prologue();
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int P = H * W;
   if (idx >= (long long)B * P) return;
@@ -314,50 +305,7 @@ __global__ void k_flow_cols(const float* __restrict__ c0, const float* __restric
 }
 int raft_flow_cols(const float* c0, const float* c1, int B, int H, int W, int pad, long long img_rows, __half* hx, __half* rhx,
                    cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_flow_cols, dim3((unsigned)(((long long)B * H * W + 255) / 256)), dim3(256), 0, s, c0, c1, B, H, W, pad, img_rows, hx, rhx));
-  PRISMA_CUDA_OK(cudaGetLastError());
-  return 0;
-}
-// ------------------------------------------------------------------------------------------------
-// SepConvGRU gate algebra (update.py:45-60) on padded rows:  rh = r * h ;  h = (1 - z) * h + z * q
-// zr: fp16 [rows][256] = [z | r] (sigmoid applied in the conv epilogue), q: fp16 [rows][128] (tanh applied).
-// ------------------------------------------------------------------------------------------------
-// The gates stay fp32 end to end (conv epilogue -> these kernels): only conv OPERANDS are fp16 in the recurrence.
-__global__ void k_gru_rh(const float* __restrict__ zr, const float* __restrict__ h_master, __half* __restrict__ rhx,
-                         long long rows) {
-  pdl_prologue();
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // rows * 32 (4 channels each)
-  if (idx >= rows * 32) return;
-  const long long row = idx >> 5;
-  const int c = (int)(idx & 31) * 4;
-  const float4 r = *reinterpret_cast<const float4*>(zr + row * 256 + 128 + c);
-  const float4 h = *reinterpret_cast<const float4*>(h_master + row * 128 + c);
-  *reinterpret_cast<uint2*>(rhx + row * 384 + c) = make_uint2(pack_half2(r.x * h.x, r.y * h.y), pack_half2(r.z * h.z, r.w * h.w));
-}
-__global__ void k_gru_update(const float* __restrict__ zr, const float* __restrict__ q, float* __restrict__ h_master,
-                             __half* __restrict__ hx, long long rows) {
-  pdl_prologue();
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= rows * 32) return;
-  const long long row = idx >> 5;
-  const int c = (int)(idx & 31) * 4;
-  const float4 z = *reinterpret_cast<const float4*>(zr + row * 256 + c);
-  const float4 qq = *reinterpret_cast<const float4*>(q + row * 128 + c);
-  float4 h = *reinterpret_cast<float4*>(h_master + row * 128 + c);
-  h.x = (1.f - z.x) * h.x + z.x * qq.x;
-  h.y = (1.f - z.y) * h.y + z.y * qq.y;
-  h.z = (1.f - z.z) * h.z + z.z * qq.z;
-  h.w = (1.f - z.w) * h.w + z.w * qq.w;
-  *reinterpret_cast<float4*>(h_master + row * 128 + c) = h;
-  *reinterpret_cast<uint2*>(hx + row * 384 + c) = make_uint2(pack_half2(h.x, h.y), pack_half2(h.z, h.w));
-}
-int raft_gru_rh(const float* zr, const float* h_master, __half* rhx, long long rows, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_gru_rh, dim3((unsigned)((rows * 32 + 255) / 256)), dim3(256), 0, s, zr, h_master, rhx, rows));
-  PRISMA_CUDA_OK(cudaGetLastError());
-  return 0;
-}
-int raft_gru_update(const float* zr, const float* q, float* h_master, __half* hx, long long rows, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_gru_update, dim3((unsigned)((rows * 32 + 255) / 256)), dim3(256), 0, s, zr, q, h_master, hx, rows));
+  k_flow_cols<<<(unsigned)(((long long)B * H * W + 255) / 256), 256, 0, s>>>(c0, c1, B, H, W, pad, img_rows, hx, rhx);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -365,7 +313,6 @@ int raft_gru_update(const float* zr, const float* q, float* h_master, __half* hx
 // coords1 += delta_flow (raft.py:133); delta: fp32 padded rows [rows][4] (cols 0,1 used)
 __global__ void k_coords_update(const float* __restrict__ delta, int B, int H, int W, int pad, long long img_rows,
                                 float* __restrict__ coords1) {
-  pdl_prologue();
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int P = H * W;
   if (idx >= (long long)B * P) return;
@@ -377,7 +324,7 @@ __global__ void k_coords_update(const float* __restrict__ delta, int B, int H, i
   coords1[(size_t)b * 2 * P + P + r] += delta[prow * 4 + 1];
 }
 int raft_coords_update(const float* delta, int B, int H, int W, int pad, long long img_rows, float* coords1, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_coords_update, dim3((unsigned)(((long long)B * H * W + 255) / 256)), dim3(256), 0, s, delta, B, H, W, pad, img_rows, coords1));
+  k_coords_update<<<(unsigned)(((long long)B * H * W + 255) / 256), 256, 0, s>>>(delta, B, H, W, pad, img_rows, coords1);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -391,7 +338,6 @@ int raft_coords_update(const float* delta, int B, int H, int W, int pad, long lo
 // ------------------------------------------------------------------------------------------------
 __global__ void k_flow_head2_gather(const float* __restrict__ u, int B, int H, int W, int pad, long long img_rows, float b0,
                                     float b1, float* __restrict__ coords1) {
-  pdl_prologue();
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int P = H * W, Wp = W + pad;
   if (idx >= (long long)B * P) return;
@@ -411,13 +357,12 @@ __global__ void k_flow_head2_gather(const float* __restrict__ u, int B, int H, i
 }
 int raft_flow_head2_gather(const float* u, int B, int H, int W, int pad, long long img_rows, float b0, float b1, float* coords1,
                            cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_flow_head2_gather, dim3((unsigned)(((long long)B * H * W + 255) / 256)), dim3(256), 0, s, u, B, H, W, pad, img_rows, b0, b1, coords1));
+  k_flow_head2_gather<<<(unsigned)(((long long)B * H * W + 255) / 256), 256, 0, s>>>(u, B, H, W, pad, img_rows, b0, b1, coords1);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
 __global__ void k_coords_init(float* __restrict__ c0, float* __restrict__ c1, int B, int H, int W) {
-  pdl_prologue();
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int P = H * W;
   if (idx >= (long long)B * P) return;
@@ -427,7 +372,7 @@ __global__ void k_coords_init(float* __restrict__ c0, float* __restrict__ c1, in
   c1[(size_t)b * 2 * P + r] = x; c1[(size_t)b * 2 * P + P + r] = y;
 }
 int raft_coords_init(float* c0, float* c1, int B, int H, int W, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_coords_init, dim3((unsigned)(((long long)B * H * W + 255) / 256)), dim3(256), 0, s, c0, c1, B, H, W));
+  k_coords_init<<<(unsigned)(((long long)B * H * W + 255) / 256), 256, 0, s>>>(c0, c1, B, H, W);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -441,7 +386,6 @@ int raft_coords_init(float* c0, float* c1, int B, int H, int W, cudaStream_t s) 
 __global__ void k_convex_upsample(const float* __restrict__ mask, const float* __restrict__ c0,
                                   const float* __restrict__ c1, int B, int H, int W, int pad, long long img_rows, int Hs,
                                   int Ws, int pad_top, int pad_left, float* __restrict__ out) {
-  pdl_prologue();
   const int b = blockIdx.y;
   const int r = blockIdx.x;  // coarse pixel
   const int y = r / W, x = r - y * W;
@@ -476,7 +420,7 @@ __global__ void k_convex_upsample(const float* __restrict__ mask, const float* _
 }
 int raft_convex_upsample(const float* mask, const float* c0, const float* c1, int B, int H, int W, int pad, long long img_rows,
                          int Hs, int Ws, int pad_top, int pad_left, float* out, cudaStream_t s) {
-  PRISMA_CUDA_OK(pdl_launch(k_convex_upsample, dim3(dim3(H * W, B)), dim3(64), 0, s, mask, c0, c1, B, H, W, pad, img_rows, Hs, Ws, pad_top, pad_left, out));
+  k_convex_upsample<<<dim3(H * W, B), 64, 0, s>>>(mask, c0, c1, B, H, W, pad, img_rows, Hs, Ws, pad_top, pad_left, out);
   PRISMA_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -19,8 +19,6 @@ int raft_cnet_split(const float* cn, int B, int H, int W, int pad, long long img
 int raft_flow_im2col(const float* c0, const float* c1, int B, int H, int W, __half* out, cudaStream_t s);
 int raft_flow_cols(const float* c0, const float* c1, int B, int H, int W, int pad, long long img_rows, __half* hx, __half* rhx,
                    cudaStream_t s);
-int raft_gru_rh(const float* zr, const float* h_master, __half* rhx, long long rows, cudaStream_t s);
-int raft_gru_update(const float* zr, const float* q, float* h_master, __half* hx, long long rows, cudaStream_t s);
 int raft_coords_update(const float* delta, int B, int H, int W, int pad, long long img_rows, float* coords1, cudaStream_t s);
 // FlowHead.conv2 as 1x1 GEMM partial products u [rows][32] (column tap*2 + out) + this nine-tap gather; coords1 += delta
 int raft_flow_head2_gather(const float* u, int B, int H, int W, int pad, long long img_rows, float b0, float b1, float* coords1,

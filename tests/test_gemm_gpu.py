@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 import torch
 
-from prisma_b200._lib import check, fptr, lib
+from prisma_b200._lib import PrismaError, check, fptr, lib
 
 pytestmark = pytest.mark.gpu
 
@@ -38,8 +38,6 @@ def _gemm(A, W, bias, act, bn):
     (2443, 3072, 1024, 0, 512),  # CTA pairs, ViT-L qkv: ragged M, many tiles per pair
     (9772, 1024, 4096, 1, 512),  # CTA pairs, 4-frame fc2 shape with gelu
     (300, 256, 200, 2, 512),     # CTA pairs: second CTA's rows partly / fully out of range, K tail
-    (37000, 128, 1920, 0, 384),  # CTA pairs with 256 x 128 tiles (the RAFT GRU q conv shape), ragged M
-    (700, 256, 320, 2, 384),     # 256 x 128 pair tiles, two column tiles, K tail
     # auto tile choice with a partial last wave -> mixed-width tail tiles (GemmArgs::tail_split)
     (29316, 1024, 192, 0, 0),    # CTA pairs: 460 pair tiles = 6 waves + 16 -> the 16 cut into 4 x 64-wide tiles
     (26624, 256, 128, 2, 0),     # CTA pairs: 104 pair tiles = 1 wave + 30 -> cut into 2 x 128-wide tiles
@@ -71,7 +69,7 @@ def test_gemm_matches_fp32_reference(M, N, K, act, bn):
 
 @pytest.mark.parametrize("M,N,K,bn", [
     (18360, 18360, 256, 0),   # RAFT correlation level 0 at 1080p x 0.75: CTA pairs, ragged M and N (N % 32 = 24)
-    (18360, 4592, 512, 0),    # level 1 (hi/lo pooled features: K = 512), N % 32 = 16
+    (18360, 4592, 512, 0),    # coarse-level size class with a longer K, N % 32 = 16
     (1000, 264, 256, 128),    # level 3 size class, single CTAs, 128-wide tiles
     (300, 520, 64, 256),      # single CTAs, 256-wide, rows of the last tile out of range
 ])
@@ -91,7 +89,7 @@ def test_gemm_tma_store_epilogue(M, N, K, bn):
 
 @pytest.mark.parametrize("M,N,K,bn", [
     (18360, 18360, 256, 0),   # RAFT correlation level 0 at 1080p x 0.75: CTA pairs, ragged M and N (N % 32 = 24)
-    (18360, 4592, 512, 0),    # level 1 (hi/lo pooled features: K = 512), N % 32 = 16
+    (18360, 4592, 512, 0),    # coarse-level size class with a longer K, N % 32 = 16
     (1000, 264, 256, 128),    # level 3 size class, single CTAs, 128-wide tiles
     (300, 520, 64, 256),      # single CTAs, 256-wide, rows of the last tile out of range
 ])
@@ -179,9 +177,9 @@ def test_gemm_tf32x3_is_fp32_class(M, N, K, bn):
     """The 3xTF32 path (kind::tf32 MMAs on [hi | lo] splits of both operands) against the exact product (float64).  The
     products are fp32-class (the dropped lo x lo term is 2^-22).  The tensor core's own fp32 ACCUMULATION truncates the aligned
     addends instead of rounding them -- with the whole K in one TMEM chain that bias measured 3e-6 .. 6e-6 of sum |a||w| on
-    B200 (growing with K; PRISMA_TF32_ACC_GROUP=0 reproduces it), i.e. only 1e-4-class results for K ~ 4600.  The kernel
-    therefore keeps a TMEM chain 4 K-blocks (16 MMAs) long and adds the partial sums in registers with round-to-nearest
-    FADDs (GemmArgs::acc_group): the error is then that of a CUDA-core fp32 GEMM."""
+    B200 (growing with K), i.e. only 1e-4-class results for K ~ 4600.  The kernel therefore keeps a TMEM chain 4 K-blocks
+    (16 MMAs) long and adds the partial sums in registers with round-to-nearest FADDs (GEMM_TF32_ACC_GROUP): the error is
+    then that of a CUDA-core fp32 GEMM."""
     rng = np.random.default_rng(M + N + K)
     A = (rng.standard_normal((M, K), dtype=np.float32) * rng.uniform(0.01, 30.0, (M, 1)).astype(np.float32))
     W = (rng.standard_normal((N, K), dtype=np.float32) / np.sqrt(K)).astype(np.float32)
@@ -194,3 +192,15 @@ def test_gemm_tf32x3_is_fp32_class(M, N, K, bn):
     err = float((np.abs(D - ref) / scale).max())
     print(f"tf32x3 {M}x{N}x{K}: max |err| / sum|a||w| = {err:.2e}, {ms.value * 1e3:.1f} us")
     assert err <= 6e-7, err
+
+
+def test_gemm_rejects_tile_widths_without_a_kernel():
+    """A requested tile width no kernel is built for is an error, never a silent substitute: 256 x 128 CTA-pair tiles
+    (force 384) on the fp16 path, and 3xTF32 tiles wider than the 128 columns its register-held running sums allow."""
+    A = np.ones((256, 64), np.float32)
+    W = np.ones((256, 64), np.float32)
+    D = np.empty((256, 256), np.float32)
+    with pytest.raises(PrismaError, match="BLOCK_N"):
+        check(lib().prisma_debug_gemm(0, fptr(A), fptr(W), None, fptr(D), 256, 256, 64, 0, 384, 1, None))
+    with pytest.raises(PrismaError, match="BLOCK_N"):
+        check(lib().prisma_debug_gemm_tf32x3(0, fptr(A), fptr(W), None, fptr(D), 256, 256, 64, 256, 1, None))

@@ -254,7 +254,7 @@ def test_solo_r101_exact_backbone_720p_reproduces_the_oracle_instances(r101_orac
     eng.close()
     # 100 convs deep the tensor core's truncating fp32 accumulate (chains of 16 MMAs between the round-to-nearest external
     # sums) shows as a uniform 1.5e-5 shrink of the FPN levels; the scores follow (measured 1.07e-4 relative, 5.5e-5 with
-    # PRISMA_TF32_ACC_GROUP=1); the instance list and all but 53 of 18.4 M mask bits are the oracle's
+    # chains of 4 MMAs); the instance list and all but 53 of 18.4 M mask bits are the oracle's
     check_instances_exact(res, scores, labels, masks, tag="r101-exact 720p", score_tol=2e-4)
 
 

@@ -1,4 +1,4 @@
-"""Sustained (power-capped) time of the encoder GEMM shapes; env PRISMA_GEMM_RASTER=m|n selects the tile walk."""
+"""Sustained (power-capped) time of the encoder GEMM shapes."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.argv = [sys.argv[0], "none"]
